@@ -14,7 +14,8 @@ HBM, e2e = the same metric through the host-buffer API (pinned H2D + kernel + D2
 roofline = algorithmic bytes / CUDA-event time against the measured HBM peak, cpu_baseline = the
 reference's per-frame CPU path (oracle port: cv2.triangulatePoints + cv2.projectPoints loop) timed
 on this box's host cores on a bounded sample.  `--impl reference` times that CPU path alone with
-all host cores.
+all host cores.  `--dump-outputs DIR` writes the arrays the timed step computed (X, err; rank 0) as .npy files: the
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -39,7 +40,8 @@ HBM_FALLBACK_GBS = 6650.0  # /opt/skills/guides/B200_PROFILING.md fallback
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, default=50, help="timed steps of the headline kernel loop (`value`, `ms_per_step`); the "
+                    "host-buffer arms time min(steps, 10) but at least 3 (their `steps`), the extra objects their own fixed counts")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--frames", type=int, default=1_000_000)
@@ -58,7 +60,12 @@ def parse():
     ap.add_argument("--e2e-chunk", type=int, default=131072, help="frames per H2D -> kernel -> D2H chunk of the host pipeline")
     ap.add_argument("--e2e-streams", type=int, default=3)
     ap.add_argument("--e2e-graph", action="store_true", help="replay the host pipeline's copies and kernels as one CUDA graph instead of enqueueing them call by call (same speed: the copies bound it)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write X.npy (T,J,3) and err.npy (V,T,J) of the last step "
+                    "(float32, rank 0) to DIR; above 32 MiB a fixed seeded sample of frames is written")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
 
 
 def workload_config(a, V):
@@ -679,6 +686,28 @@ def fusion_cpu_rate(frames=600):
     return frames / (time.perf_counter() - t0)
 
 
+DUMP_BYTES = 32 << 20
+
+
+def dump_outputs(out_dir, outs):
+    """Write the arrays the timed step returns (X, err) as float32 .npy files, so that two builds run with the same
+    arguments can be compared output for output.  Above DUMP_BYTES the same seeded sample of frames is taken every run."""
+    import torch
+
+    X, err = outs["X"], outs["err"]
+    T = X.shape[0]
+    n = min(T, DUMP_BYTES // ((X[0].numel() + err[:, 0].numel()) * 4))
+    if n == 0:
+        raise SystemExit(f"--dump-outputs: one frame of X and err is larger than {DUMP_BYTES} bytes")
+    if n < T:
+        idx = torch.from_numpy(np.sort(np.random.default_rng(0).choice(T, n, replace=False))).to(X.device)
+        X, err = X[idx], err[:, idx]
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    np.save(d / "X.npy", X.cpu().numpy())
+    np.save(d / "err.npy", err.cpu().numpy())
+
+
 def run_ours(a, out_fd=1):
     import torch
     import torch.distributed as dist
@@ -763,6 +792,8 @@ def run_ours(a, out_fd=1):
         # what the host side gives with all ranks copying at once: the ceiling of the end-to-end number at this N
         link = hostlink.measure_link(dev, barrier=barrier)
 
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, outs)  # the host-buffer arm writes its own buffers: outs still holds the last timed step
     t_k = torch.tensor([kernel_ms, e2e_ms, e2e_full_ms], dtype=torch.float64, device=dev)
     t_l = torch.tensor([link["h2d_alone"], link["d2h_alone"], link["both_each"]], dtype=torch.float64, device=dev)
     if world > 1:

@@ -22,6 +22,8 @@ tests only ever read the .npz files.  Golden sets (SURVEY.md section 8c):
   G6  LM history of oracle/lm.py on BASELINE configs 3 and 5 at reduced T, with the REFERENCE's
       reprojection_loss evaluated at the initial and final state of each solve (pins the cost the
       LM minimises; the trajectory itself has no reference implementation - "parity unpinned")
+  reference_signatures.json  parameter names and scalar defaults of the reference functions the drop-in shims
+      stand in for (--only-signatures)
 """
 from __future__ import annotations
 
@@ -451,8 +453,24 @@ def g12():
     print("g12 written:", {n: (out[f"{n}_cost"][0], out[f"{n}_final_cost"], out[f"{n}_ref_loss_final"]) for n in lm_reg.G12_CASES})
 
 
+def signatures():
+    """Parameter names and scalar defaults of every reference function listed in reference_signatures.json, re-read
+    from the checkout (tests/test_dropin_cpu.py holds the drop-in shims to them)."""
+    import json
+
+    f = OUT / "reference_signatures.json"
+    rec = json.loads(f.read_text())
+    for module, funcs in rec.items():
+        ref = ref_import.load(module)
+        for fn in funcs:
+            funcs[fn] = ref_import.signature_record(getattr(ref, fn))
+    f.write_text(json.dumps(rec, indent=1) + "\n")
+
+
 def main():
     OUT.mkdir(parents=True, exist_ok=True)
+    if "--only-signatures" in sys.argv:
+        return signatures()
     if "--only-g12" in sys.argv:
         return g12()
     if "--only-g11" in sys.argv:
@@ -470,6 +488,7 @@ def main():
     g2()
     g3_g4()
     g6()
+    signatures()
     for f in sorted(OUT.glob("*.npz")):
         print(f.name, f.stat().st_size)
 

@@ -1,9 +1,9 @@
-"""Import the reference's own hot-path modules from /root/reference (authoring container only).
+"""Import the reference's own hot-path modules from a checkout of it (SKA_REFERENCE_ROOT).
 
 The viz imports the reference pulls at module import (matplotlib, plotly; triangulation/vis/
-pose_visualization.py:9,17-19 and vggt/vis/pose_visualization.py:10-11) are not installed, so dummy
-sys.modules entries are inserted first (SURVEY.md section 8c).  Used by make_golden.py and by the
-tests marked ``needs_reference``; nothing that runs on the GPU box may call this.
+pose_visualization.py:9,17-19 and vggt/vis/pose_visualization.py:10-11) may not be installed, so dummy
+sys.modules entries are inserted first (SURVEY.md section 8c).  Used by make_golden.py and by tests
+that compare with the checkout when one is present; signature_record() needs no checkout.
 """
 from __future__ import annotations
 
@@ -45,6 +45,23 @@ def _install_stubs():
                 importlib.import_module(name)
             except Exception:
                 sys.modules[name] = _Anything(name)
+
+
+def signature_record(fn) -> list:
+    """The parameters of `fn` in order, as JSON-ready dicts: {"name"} when it has no default, {"name", "default"} when the
+    default is an int / float / str / bool / None, {"name", "default_is_object": True} for any other default."""
+    import inspect
+
+    out = []
+    for p in inspect.signature(fn).parameters.values():
+        d = p.default
+        if d is inspect.Parameter.empty:
+            out.append({"name": p.name})
+        elif isinstance(d, (int, float, str, bool, type(None))):
+            out.append({"name": p.name, "default": d})
+        else:
+            out.append({"name": p.name, "default_is_object": True})
+    return out
 
 
 def load(module: str):
