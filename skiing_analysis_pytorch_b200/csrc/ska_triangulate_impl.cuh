@@ -15,6 +15,9 @@
 //           triangulation/reproject.py:49-83,243-244 (file:line in the reference checkout).
 #pragma once
 #include <cuda_runtime.h>
+#ifdef SKA_CTA_WAIT_CLOCKS
+#include <cstdio>
+#endif
 
 #include "ska_internal.h"
 #include "ska_tri_point.cuh"
@@ -251,10 +254,12 @@ __global__ void __launch_bounds__(kBlock, MINB) tri_kernel(const __grid_constant
 // the two points as ONE packed (F2 -> FFMA2) computation.  Consumers issue no global loads and no load addressing;
 // the producer costs ~2 instructions per tile (the first form of this kernel fed every consumer warp from its own
 // producer lane: 22 serialised single-lane copies per group, ~40 issue slots per tile).
+// (16 consumer warps - four per scheduler - with lane 0 of warp 0 as the producer, polling `empty` between its own
+// tiles, was built and measured slower: 0.157 against 0.145 ms on config 2, profiles/r03_tri_cta_config2_bounds.log.)
 //
 // The arithmetic per pair is fast_stage<> (normal matrix, one LDL^T, secular step, certificate) -> ONE warp vote ->
 // final row residuals -> scoring.  A warp in which any point fails the certificate (rare: near-degenerate geometry,
-// non-finite input) finishes its tile in tri_pair_cold (noinline: general secular iteration + fp64 Jacobi), so the
+// non-finite input) finishes its tile in tri_pair_cold (general secular iteration + fp64 Jacobi), so the
 // hot loop carries none of that state.  X leaves through a per-warp staging buffer as 128-bit stores, the per-view
 // error as 64-bit stores.
 #ifdef SKA_PLAIN_STORES  // measurement variant: default-policy stores instead of st.global.cs
@@ -305,67 +310,84 @@ constexpr int kColdCap = 32;  // per-warp list of tiles deferred to the cold loo
 
 // (A group of NW + 1 tiles whose extra tile rotates over the consumer warps that share the producer warp's scheduler - so
 // that every scheduler computes four tiles per group - was measured slower: 0.162 against 0.149 ms on config 2.)
-template <int NW>
-struct CtaGroup {
-  static constexpr int kTiles = NW;
-};
-
 template <int V, int NW, bool CONF, int STAGES>
 struct CtaSmem {  // dynamic shared-memory layout of tri_kernel_cta
-  static constexpr int GT = CtaGroup<NW>::kTiles;
-  static constexpr int kViewK = GT * kWarpPts * 2;           // floats of one view's keypoints in a stage
-  static constexpr int kViewC = CONF ? GT * kWarpPts : 0;    // ... confidences
+  static constexpr int kViewK = NW * kWarpPts * 2;           // floats of one view's keypoints in a stage
+  static constexpr int kViewC = CONF ? NW * kWarpPts : 0;    // ... confidences
   static constexpr int kKptFloats = V * kViewK;
   static constexpr int kStageFloats = kKptFloats + V * kViewC;
   static constexpr size_t oX = (size_t)STAGES * kStageFloats * sizeof(float);
   static constexpr size_t oFull = oX + (size_t)NW * kWarpPts * 3 * sizeof(float);
   static constexpr size_t oEmpty = oFull + (size_t)STAGES * sizeof(uint64_t);
-  static constexpr size_t oCold = oEmpty + (size_t)STAGES * sizeof(uint64_t);
+  static constexpr size_t oState = oEmpty + (size_t)STAGES * sizeof(uint64_t);
+  static constexpr size_t oCold = oState + (size_t)NW * 2 * sizeof(uint32_t);
   static constexpr size_t bytes = oCold + (size_t)NW * kColdCap * sizeof(uint32_t);
 };
 
-// The rare tile: general secular iteration / fp64 fallback for the lane's pair (the general tri_points<>), results
-// written where the hot path writes them.  Runs in the deferred cold loop of tri_kernel_cta, outside the hot loop.
+// The rare tile: general secular iteration / fp64 fallback for each point of the lane's pair (the general tri_points<>
+// one point at a time: the scalar kernel's arithmetic, in half the registers of the packed pair), results written where
+// the hot path writes them.  Runs in the deferred cold loop of tri_kernel_cta, outside the hot loop.
 template <int V, bool CONF, int DIST, bool SAMEK>
 __device__ __forceinline__ void tri_pair_cold(const TriParams<V>& prm, uint32_t i0, float* sx6) {
-  constexpr int PTS = 2;
-  float u[PTS][V], v[PTS][V], w2[PTS][V], du[PTS][V], dv[PTS][V], X[PTS][3];
-  uint8_t stt[PTS];
+#pragma unroll 1
+  for (uint32_t i = i0; i < i0 + 2; ++i) {
+    float u[1][V], v[1][V], w2[1][V], du[1][V], dv[1][V], X[1][3];
+    uint8_t stt[1];
 #pragma unroll
-  for (int k = 0; k < V; ++k) {  // the stage was handed back: the pair is read again from global memory
-    const float4 q = *reinterpret_cast<const float4*>(prm.kpts + (int64_t)k * prm.k_sV + 2 * (int64_t)i0);
-    u[0][k] = q.x; v[0][k] = q.y; u[1][k] = q.z; v[1][k] = q.w;
-    float2 cf = make_float2(1.f, 1.f);
-    if (CONF) cf = *reinterpret_cast<const float2*>(prm.conf + (int64_t)k * prm.c_sV + i0);
-    w2[0][k] = CONF ? (prm.weight_sqrt ? cf.x : cf.x * cf.x) : 1.0f;
-    w2[1][k] = CONF ? (prm.weight_sqrt ? cf.y : cf.y * cf.y) : 1.0f;
-  }
-  PointSource src;
-  src.kpts = prm.kpts + 2 * (int64_t)i0;
-  src.conf = (CONF && prm.conf != nullptr) ? prm.conf + i0 : nullptr;
-  src.k_sV = prm.k_sV;
-  src.c_sV = prm.c_sV;
-  src.weight_sqrt = prm.weight_sqrt;
-  tri_points<V, PTS, CONF, DIST, kSolverSecular, 1, SAMEK>(prm.cam, prm.P64, prm.c[0], prm.c[1], prm.c[2], u, v, w2, src, X, du, dv, stt);
-#pragma unroll
-  for (int k = 0; k < V; ++k) {
-    if (prm.err != nullptr) {
-      const float e0 = sqrt_fast(fmaf(du[0][k], du[0][k], dv[0][k] * dv[0][k]));
-      const float e1 = sqrt_fast(fmaf(du[1][k], du[1][k], dv[1][k] * dv[1][k]));
-      __stcs(reinterpret_cast<float2*>(prm.err + (int64_t)k * prm.c_sV + i0), make_float2(e0, e1));
+    for (int k = 0; k < V; ++k) {  // the stage was handed back: the point is read again from global memory
+      const float2 q = *reinterpret_cast<const float2*>(prm.kpts + (int64_t)k * prm.k_sV + 2 * (int64_t)i);
+      u[0][k] = q.x;
+      v[0][k] = q.y;
+      const float cf = CONF ? prm.conf[(int64_t)k * prm.c_sV + i] : 1.0f;
+      w2[0][k] = CONF ? (prm.weight_sqrt ? cf : cf * cf) : 1.0f;
     }
-    if (prm.proj != nullptr)
-      __stcs(reinterpret_cast<float4*>(prm.proj + (int64_t)k * prm.k_sV + 2 * (int64_t)i0),
-             make_float4(u[0][k] + du[0][k], v[0][k] + dv[0][k], u[1][k] + du[1][k], v[1][k] + dv[1][k]));
+    PointSource src;
+    src.kpts = prm.kpts + 2 * (int64_t)i;
+    src.conf = (CONF && prm.conf != nullptr) ? prm.conf + i : nullptr;
+    src.k_sV = prm.k_sV;
+    src.c_sV = prm.c_sV;
+    src.weight_sqrt = prm.weight_sqrt;
+    tri_points<V, 1, CONF, DIST, kSolverSecular, 1, SAMEK>(prm.cam, prm.P64, prm.c[0], prm.c[1], prm.c[2], u, v, w2, src, X, du, dv, stt);
+#pragma unroll
+    for (int k = 0; k < V; ++k) {
+      if (prm.err != nullptr) __stcs(prm.err + (int64_t)k * prm.c_sV + i, sqrt_fast(fmaf(du[0][k], du[0][k], dv[0][k] * dv[0][k])));
+      if (prm.proj != nullptr)
+        __stcs(reinterpret_cast<float2*>(prm.proj + (int64_t)k * prm.k_sV + 2 * (int64_t)i), make_float2(u[0][k] + du[0][k], v[0][k] + dv[0][k]));
+    }
+    if (prm.status != nullptr) prm.status[i] = stt[0];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) sx6[(i - i0) * 3 + k] = X[0][k];
   }
-  if (prm.status != nullptr) *reinterpret_cast<uchar2*>(prm.status + i0) = make_uchar2(stt[0], stt[1]);
-#pragma unroll
-  for (int p = 0; p < PTS; ++p)
-#pragma unroll
-    for (int k = 0; k < 3; ++k) sx6[p * 3 + k] = X[p][k];
 }
 
+// One group's bulk copies into `stage`: one per view (plus one per view of confidences), `full` expects their bytes.
+template <int V, bool CONF, int NW, int STAGES>
+__device__ __forceinline__ void cta_issue(const TriParams<V>& prm, float* stage, uint64_t* full, uint32_t g, uint32_t n_wt) {
+  using L = CtaSmem<V, NW, CONF, STAGES>;
+  const uint32_t t0 = g * NW;
+  const uint32_t nt = (n_wt - t0 < (uint32_t)NW) ? (n_wt - t0) : (uint32_t)NW;
+#ifdef SKA_CTA_L2_WINDOW  // measurement variant: copy from a 32-group window that stays in L2 (same instructions, no HBM reads)
+  const uint32_t ts = (g % 32u) * NW;
+#else
+  const uint32_t ts = t0;
+#endif
+  mbar_expect_tx(full, (uint32_t)V * nt * (uint32_t)(kWarpPts * (CONF ? 12 : 8)));
+#pragma unroll
+  for (int k = 0; k < V; ++k) {
+    bulk_g2s(stage + k * L::kViewK, prm.kpts + (int64_t)k * prm.k_sV + (int64_t)ts * (kWarpPts * 2), nt * (kWarpPts * 8), full);
+    if (CONF)
+      bulk_g2s(stage + L::kKptFloats + k * L::kViewC, prm.conf + (int64_t)k * prm.c_sV + (int64_t)ts * kWarpPts, nt * (kWarpPts * 4), full);
+  }
+}
+
+#ifdef SKA_CTA_WAIT_CLOCKS  // measurement variant: clock64() spent waiting on `full`, summed over the launch and printed
+__device__ unsigned long long g_cta_clocks[4];
+#endif
+
 // LEAN: the common output set (X and err, no proj / status, 16-byte aligned X) compiled without pointer tests.
+//
+// Loop state is one counter: k = how many of this CTA's groups were taken; the group is blockIdx.x + k * gridDim.x, its
+// stage k % STAGES, the phase parity (k / STAGES) & 1.
 template <int V, bool CONF, int DIST, int NW, int STAGES, bool SAMEK, bool LEAN>
 __global__ void __maxnreg__(SKA_CTA_MAXREG) tri_kernel_cta(const __grid_constant__ TriParams<V> prm) {
   using L = CtaSmem<V, NW, CONF, STAGES>;
@@ -374,14 +396,15 @@ __global__ void __maxnreg__(SKA_CTA_MAXREG) tri_kernel_cta(const __grid_constant
   float(*sX)[kWarpPts * 3] = reinterpret_cast<float(*)[kWarpPts * 3]>(cta_smem + L::oX);
   uint64_t* sFull = reinterpret_cast<uint64_t*>(cta_smem + L::oFull);
   uint64_t* sEmpty = reinterpret_cast<uint64_t*>(cta_smem + L::oEmpty);
+  uint32_t* sState = reinterpret_cast<uint32_t*>(cta_smem + L::oState);  // per warp: k, n_cold during the cold loop
   uint32_t(*sCold)[kColdCap] = reinterpret_cast<uint32_t(*)[kColdCap]>(cta_smem + L::oCold);
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const uint32_t n_wt = (uint32_t)prm.n_tiles;             // whole 64-point tiles
-  constexpr int GT = CtaGroup<NW>::kTiles;
-  const uint32_t n_groups = (n_wt + GT - 1) / GT;
+  const uint32_t n_wt = (uint32_t)prm.n_tiles;  // whole 64-point tiles
+  const uint32_t n_groups = (n_wt + NW - 1) / NW;
+  const uint32_t n_mine = (n_groups - blockIdx.x + gridDim.x - 1) / gridDim.x;  // groups of this CTA (grid <= n_groups)
   if (threadIdx.x < STAGES) {
     mbar_init(sFull + threadIdx.x, 1);
-    mbar_init(sEmpty + threadIdx.x, GT);  // one arrival per tile
+    mbar_init(sEmpty + threadIdx.x, NW);  // one arrival per tile
   }
   asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
@@ -390,70 +413,69 @@ __global__ void __maxnreg__(SKA_CTA_MAXREG) tri_kernel_cta(const __grid_constant
   if (warp == NW) {
     // ---------------------------------------------------------------- producer: one thread
     if (lane == 0) {
-      int st = 0;
-      uint32_t round = 0;  // how many times the ring wrapped
-      for (uint32_t g = blockIdx.x; g < n_groups; g += gridDim.x) {
-        if (round > 0) mbar_wait(sEmpty + st, (round - 1) & 1u);  // every tile of the stage's previous group was taken
-        const uint32_t t0 = g * GT;
-        const uint32_t nt = (n_wt - t0 < (uint32_t)GT) ? (n_wt - t0) : (uint32_t)GT;
-        float* stage = sK + (size_t)st * L::kStageFloats;
-        mbar_expect_tx(sFull + st, (uint32_t)V * nt * (uint32_t)(kWarpPts * (CONF ? 12 : 8)));
-#pragma unroll
-        for (int k = 0; k < V; ++k) {
-          bulk_g2s(stage + k * L::kViewK, prm.kpts + (int64_t)k * prm.k_sV + (int64_t)t0 * (kWarpPts * 2), nt * (kWarpPts * 8), sFull + st);
-          if (CONF)
-            bulk_g2s(stage + L::kKptFloats + k * L::kViewC, prm.conf + (int64_t)k * prm.c_sV + (int64_t)t0 * kWarpPts, nt * (kWarpPts * 4),
-                     sFull + st);
-        }
-        if (++st == STAGES) {
-          st = 0;
-          ++round;
-        }
+      for (uint32_t p = 0; p < n_mine; ++p) {
+        if (p >= STAGES) mbar_wait(sEmpty + p % STAGES, (p / STAGES - 1) & 1u);  // every tile of the stage's previous group was taken
+        cta_issue<V, CONF, NW, STAGES>(prm, sK + (size_t)(p % STAGES) * L::kStageFloats, sFull + p % STAGES, blockIdx.x + p * gridDim.x, n_wt);
       }
     }
     return;
   }
 
   // ------------------------------------------------------------------ consumer warps
-  int st = 0;
-  uint32_t par = 0;
   float* sx = sX[warp];
   uint32_t* cold = sCold[warp];  // tiles of this warp that failed the certificate vote, finished after the hot loop
   const float cx = prm.c[0], cy = prm.c[1], cz = prm.c[2];
-  uint32_t g = blockIdx.x;
+#ifdef SKA_CTA_WAIT_CLOCKS
+  unsigned long long wait_clk = 0, n_hot = 0;
+  const long long clk_start = clock64();
+#endif
+  uint32_t k = 0;
   for (;;) {
     uint32_t n_cold = 0;
     // ---- hot loop: certified tiles only
-    while (g < n_groups && n_cold < (uint32_t)kColdCap) {
-      const uint32_t slot = (uint32_t)warp;
-      const uint32_t wt = g * GT + slot;
+    while (k < n_mine && n_cold < (uint32_t)kColdCap) {
+      const uint32_t st = k % STAGES;
+      const uint32_t wt = (blockIdx.x + k * gridDim.x) * NW + (uint32_t)warp;
       if (wt >= n_wt) {  // last, partial group: nothing follows for this CTA
-        g = n_groups;
+        k = n_mine;
         break;
       }
-      mbar_wait(sFull + st, par);
+#ifdef SKA_CTA_WAIT_CLOCKS
+      const long long w0 = clock64();
+      mbar_wait(sFull + st, (k / STAGES) & 1u);
+      wait_clk += clock64() - w0;
+      ++n_hot;
+#else
+      mbar_wait(sFull + st, (k / STAGES) & 1u);
+#endif
       const float* stage = sK + (size_t)st * L::kStageFloats;
       const uint32_t i0 = wt * kWarpPts + 2u * lane;
       F2 ut[V], vt[V], w2[V];
 #pragma unroll
-      for (int k = 0; k < V; ++k) {
-        const float4 q = *reinterpret_cast<const float4*>(stage + k * L::kViewK + slot * (kWarpPts * 2) + 4 * lane);
-        ut[k] = mk2(q.x, q.z);
-        vt[k] = mk2(q.y, q.w);
+      for (int v = 0; v < V; ++v) {
+        const float4 q = *reinterpret_cast<const float4*>(stage + v * L::kViewK + warp * (kWarpPts * 2) + 4 * lane);
+        ut[v] = mk2(q.x, q.z);
+        vt[v] = mk2(q.y, q.w);
         if (CONF) {
-          const float2 cf = *reinterpret_cast<const float2*>(stage + L::kKptFloats + k * L::kViewC + slot * kWarpPts + 2 * lane);
-          w2[k] = prm.weight_sqrt ? mk2(cf.x, cf.y) : mk2(cf.x * cf.x, cf.y * cf.y);
+          const float2 cf = *reinterpret_cast<const float2*>(stage + L::kKptFloats + v * L::kViewC + warp * kWarpPts + 2 * lane);
+          w2[v] = prm.weight_sqrt ? mk2(cf.x, cf.y) : mk2(cf.x * cf.x, cf.y * cf.y);
         } else {
-          w2[k] = mk2(1.f, 1.f);
+          w2[v] = mk2(1.f, 1.f);
         }
       }
-      __syncwarp();                               // every lane holds its pair in registers
-      if (lane == 0) mbar_arrive(sEmpty + st);    // this tile's share of the stage goes back to the producer
-      g += gridDim.x;
-      if (++st == STAGES) {
-        st = 0;
-        par ^= 1u;
+      __syncwarp();                             // every lane holds its pair in registers
+      if (lane == 0) mbar_arrive(sEmpty + st);  // this tile's share of the stage goes back to the producer
+      ++k;
+#ifdef SKA_CTA_NO_MATH  // measurement variant: the staging, the vote and the stores without the arithmetic
+      F2 du[V], dv[V];
+#pragma unroll
+      for (int v = 0; v < V; ++v) {
+        du[v] = ut[v];
+        dv[v] = vmul(vt[v], w2[v]);
       }
+      const F2 Y0 = ut[0], Y1 = vt[0], Y2 = ut[V - 1];
+      if (!__all_sync(0xffffffffu, Y0.x == Y0.x || Y0.y != Y0.y)) continue;
+#else
       F2 a[V][4], b[V][4];
       Sym4T<F2> M;
       FastStage<F2> fs;
@@ -468,19 +490,21 @@ __global__ void __maxnreg__(SKA_CTA_MAXREG) tri_kernel_cta(const __grid_constant
       F2 ra[V], rb[V], du[V], dv[V];
       row_residuals<V, F2>(a, b, fs.y0, fs.y1, fs.y2, ra, rb);
       score_views<V, DIST, SAMEK, F2>(prm.cam, fs.y0, fs.y1, fs.y2, ra, rb, ut, vt, du, dv);
+      const F2 Y0 = fs.y0, Y1 = fs.y1, Y2 = fs.y2;
+#endif
 #pragma unroll
-      for (int k = 0; k < V; ++k) {
+      for (int v = 0; v < V; ++v) {
         if (LEAN || prm.err != nullptr) {
-          const F2 e = sqrt_fast(vfma(du[k], du[k], vmul(dv[k], dv[k])));
-          SKA_ST(reinterpret_cast<float2*>(prm.err + (int64_t)k * prm.c_sV + i0), make_float2(e.x, e.y));
+          const F2 e = sqrt_fast(vfma(du[v], du[v], vmul(dv[v], dv[v])));
+          SKA_ST(reinterpret_cast<float2*>(prm.err + (int64_t)v * prm.c_sV + i0), make_float2(e.x, e.y));
         }
         if (!LEAN && prm.proj != nullptr) {
-          const F2 pu = vadd(ut[k], du[k]), pv = vadd(vt[k], dv[k]);
-          SKA_ST(reinterpret_cast<float4*>(prm.proj + (int64_t)k * prm.k_sV + 2 * (int64_t)i0), make_float4(pu.x, pv.x, pu.y, pv.y));
+          const F2 pu = vadd(ut[v], du[v]), pv = vadd(vt[v], dv[v]);
+          SKA_ST(reinterpret_cast<float4*>(prm.proj + (int64_t)v * prm.k_sV + 2 * (int64_t)i0), make_float4(pu.x, pv.x, pu.y, pv.y));
         }
       }
       if (!LEAN && prm.status != nullptr) *reinterpret_cast<uchar2*>(prm.status + i0) = make_uchar2(0, 0);
-      const F2 X0 = vadd(fs.y0, cx), X1 = vadd(fs.y1, cy), X2 = vadd(fs.y2, cz);
+      const F2 X0 = vadd(Y0, cx), X1 = vadd(Y1, cy), X2 = vadd(Y2, cz);
       *reinterpret_cast<float2*>(sx + lane * 6) = make_float2(X0.x, X1.x);
       *reinterpret_cast<float2*>(sx + lane * 6 + 2) = make_float2(X2.x, X0.y);
       *reinterpret_cast<float2*>(sx + lane * 6 + 4) = make_float2(X1.y, X2.y);
@@ -496,10 +520,17 @@ __global__ void __maxnreg__(SKA_CTA_MAXREG) tri_kernel_cta(const __grid_constant
       }
       __syncwarp();  // sx is rewritten next iteration
     }
-    // ---- cold loop (rare): the tiles the vote rejected, with the general per-point code
+    // ---- cold loop (rare): the tiles the vote rejected, with the general per-point code.  The loop state waits in
+    // shared memory (volatile: kept out of the registers the general solver needs, instead of a spill slot that the
+    // hot loop would store to on every tile).
+    volatile uint32_t* wstate = sState + 2 * warp;
+    if (lane == 0) {
+      wstate[0] = k;
+      wstate[1] = n_cold;
+    }
     __syncwarp();
 #pragma unroll 1
-    for (uint32_t ci = 0; ci < n_cold; ++ci) {
+    for (uint32_t ci = 0; ci < wstate[1]; ++ci) {
       const uint32_t wt = cold[ci];
       tri_pair_cold<V, CONF, DIST, SAMEK>(prm, wt * kWarpPts + 2u * lane, sx + lane * 6);
       __syncwarp();
@@ -513,13 +544,29 @@ __global__ void __maxnreg__(SKA_CTA_MAXREG) tri_kernel_cta(const __grid_constant
       }
       __syncwarp();
     }
-    if (g >= n_groups) break;
+    k = wstate[0];
+    if (k >= n_mine) break;
   }
+#ifdef SKA_CTA_WAIT_CLOCKS
+  if (lane == 0) {
+    atomicAdd(&g_cta_clocks[0], wait_clk);
+    atomicAdd(&g_cta_clocks[1], n_hot);
+    atomicAdd(&g_cta_clocks[2], (unsigned long long)(clock64() - clk_start));
+    __threadfence();
+    if (atomicAdd(&g_cta_clocks[3], 1ull) == (unsigned long long)gridDim.x * NW - 1) {  // the last consumer warp of the launch
+      const unsigned long long w = g_cta_clocks[0], n = g_cta_clocks[1], t = g_cta_clocks[2];
+      printf("tri_kernel_cta wait clocks: %llu tiles, full-barrier wait %.1f cycles/tile, warp lifetime %.1f cycles/tile (%.1f %% waiting)\n", n,
+             (double)w / n, (double)t / n, 100.0 * w / t);
+      for (int i = 0; i < 4; ++i) g_cta_clocks[i] = 0;
+    }
+  }
+#endif
 }
 
 template <int V, bool CONF, int DIST, bool SAMEK, bool LEAN>
 static cudaError_t launch_cta_impl(TriParams<V>& prm, cudaStream_t stream) {
-  constexpr int NW = SKA_CTA_WARPS, STAGES = SKA_CTA_STAGES, BLOCK = 32 * (NW + 1);
+  // with confidences a stage is 22.5 KB: the deeper-ring measurement variants keep 8 of them
+  constexpr int NW = SKA_CTA_WARPS, STAGES = (CONF && SKA_CTA_STAGES > 8) ? 8 : SKA_CTA_STAGES, BLOCK = 32 * (NW + 1);
   auto kern = tri_kernel_cta<V, CONF, DIST, NW, STAGES, SAMEK, LEAN>;
   constexpr size_t smem = CtaSmem<V, NW, CONF, STAGES>::bytes;
   static_assert(smem <= 227 * 1024, "tri_kernel_cta staging does not fit the SM's shared memory");
@@ -530,8 +577,7 @@ static cudaError_t launch_cta_impl(TriParams<V>& prm, cudaStream_t stream) {
   if (ce != cudaSuccess) return ce;
   ce = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);  // idempotent
   if (ce != cudaSuccess) return ce;
-  constexpr int GT = CtaGroup<NW>::kTiles;
-  const int64_t n_groups = (prm.n_tiles + GT - 1) / GT;
+  const int64_t n_groups = (prm.n_tiles + NW - 1) / NW;
   int64_t grid = sms;  // one persistent CTA per SM
   if (grid > n_groups) grid = n_groups;
   kern<<<(unsigned)grid, BLOCK, smem, stream>>>(prm);

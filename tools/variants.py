@@ -18,6 +18,13 @@ VARIANTS = {
     "A": [],
     "B": ["-DSKA_FR_WARPS=10", "-DSKA_FR_PRODUCERS=2", "-DSKA_FR_STAGES=4"],
     "C": ["-DSKA_FR_STAGES=6"],
+    # tri_kernel_cta on config 2 (tools/tri_cta_bounds.py): ring depth, and three builds that exist only to be measured
+    "cta_s6": ["-DSKA_CTA_STAGES=6"],
+    "cta_s8": ["-DSKA_CTA_STAGES=8"],
+    "cta_s12": ["-DSKA_CTA_STAGES=12"],
+    "cta_l2": ["-DSKA_CTA_L2_WINDOW"],
+    "cta_nomath": ["-DSKA_CTA_NO_MATH"],
+    "cta_clocks": ["-DSKA_CTA_WAIT_CLOCKS"],
 }
 LIBDIR = ROOT / "skiing_analysis_pytorch_b200" / "lib"
 
