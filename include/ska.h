@@ -135,7 +135,7 @@ int ska_project_points_f64(const double* d_X, int64_t T, int32_t J, int32_t C, c
                            const double* d_t, int64_t t_frame_stride, const double* d_K, int64_t K_frame_stride,
                            double* d_out, void* stream);
 /* reprojection_loss  loss.py:90-94, value and analytic gradient in one pass over the observations.
- * d_sums[4] (fp64): [sum conf |proj - x2d|^2, sum conf, #clamped observations, 0];
+ * d_sums[4] (fp64): [sum conf |proj - x2d|^2, sum conf, #clamped observations, reserved (not written)];
  *                   loss = w * d_sums[0] / (d_sums[1] + 1e-6).
  * d_gX (T,J,3), d_gR / d_gt / d_gK shaped like d_R / d_t / d_K: nullable; UNSCALED gradients
  * sum conf J^T e - multiply by 2 w / (d_sums[1] + 1e-6) (what torch.autograd derives from loss.py).

@@ -224,6 +224,13 @@ class _CameraCentre(torch.autograd.Function):
         return gR.reshape(Rs).to(Rd), gt.sum_to_size(ts).to(td) if gt.shape != ts else gt.to(td)
 
 
+def _mean(w, total, count, dt):
+    """``w * total / count``; with no term (count 0) torch's mean of an empty tensor: nan, and a zero gradient."""
+    if count == 0:
+        return (w * total * 0.0 + float("nan")).to(dt)
+    return (w * total / count).to(dt)
+
+
 class _RawSum(torch.autograd.Function):
     """Generic wrapper: `launch(grads_wanted) -> (sum tensor (fp64, 0-dim), [unscaled grads])`."""
 
@@ -262,7 +269,7 @@ def camera_smooth_loss(R, t, w=1e-2):
         return s[0].clone(), [gR, gt]
 
     total = _RawSum.apply(launch, Rc, tc)
-    return (w * total / count).to(dt)  # mean of an empty tensor is nan, like torch
+    return _mean(w, total, count, dt)
 
 
 def baseline_reg_loss(R, t, w=1e-2):
@@ -354,4 +361,4 @@ def pose_temporal_loss(X3d, w=1e-2):
         return s[0].clone(), [gX]
 
     total = _RawSum.apply(launch, Xc)
-    return (w * total / (max(T - 1, 0) * J * 3)).to(dt)
+    return _mean(w, total, max(T - 1, 0) * J * 3, dt)
