@@ -26,7 +26,9 @@ BA_CTRL_DOUBLES = 16
 BA_HIST_DOUBLES = 8
 BA_RED2_DOUBLES = 4
 BA_CTRL_LAMBDA, BA_CTRL_NU, BA_CTRL_SUMCONF, BA_CTRL_CUR, BA_CTRL_ITER = 0, 1, 2, 3, 4
+BA_CTRL_PREDCAM, BA_CTRL_OK = 5, 6  # written by the solve: camera part of the predicted decrease; 1 if the reduced system was positive definite
 BA_CTRL_COST, BA_CTRL_ACCEPTED = 7, 8
+BA_CTRL_PRIOR_CUR, BA_CTRL_PRIOR_TRIAL = 9, 10  # calibrating BA, written by the solve: intrinsics-prior cost at the current / trial cameras
 BA_FORCE_WIDE = 1
 BA_TENSOR_CORE = 2
 
