@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define SKA_ABI_VERSION 8
+#define SKA_ABI_VERSION 9
 
 #define SKA_OK 0
 #define SKA_EINVAL -1       /* null pointer / bad size / bad enum */
@@ -192,6 +192,17 @@ int ska_baseline_reg_f64(const double* d_R, const double* d_t, int64_t T, int32_
  * Marquardt damping lam*diag(H) on both blocks; Schur complement onto the cameras; Cholesky;
  * back-substitution; accept iff the cost decreases; Nielsen gain-ratio damping update.
  *
+ * Robust loss (SkaBaProblem.loss / loss_scale; DESIGN.md section 5): with s = |pi_c(X) - x2d|^2 in px^2 and d > 0 the scale
+ * in pixels, the cost becomes F = sum conf/(sum conf + 1e-6) rho(s) with
+ *   SKA_BA_LOSS_L2      rho = s                                       omega = 1
+ *   SKA_BA_LOSS_HUBER   rho = s if s <= d^2, else 2 d sqrt(s) - d^2   omega = 1 if s <= d^2, else d / sqrt(s)
+ *   SKA_BA_LOSS_CAUCHY  rho = d^2 ln(1 + s / d^2)                     omega = 1 / (1 + s / d^2)
+ * and the step is iteratively reweighted Gauss-Newton: every sum above uses the weight conf * omega(s), with omega
+ * evaluated at the current state and not differentiated (the gradient is still exactly half that of F, so the gain
+ * ratio and the accept rule keep their meaning).  A depth-clamped observation is weighted by omega of its error.  Huber
+ * computes an inlier's rho and omega with the L2 expressions: a solve with every residual inside d is bit-identical to
+ * L2.  The reduced-system layout does not change.  SKA_BA_TENSOR_CORE with a robust loss returns SKA_EUNSUPPORTED.
+ *
  * One LM trial = ska_ba_linearize_f32 -> [all-reduce d_red over ranks] -> ska_ba_solve_f64 ->
  * ska_ba_backsub_f32 -> [all-reduce d_red2] -> ska_ba_control_f64.  Nothing synchronises with the host;
  * the sequence can be captured in a CUDA graph.  All state lives in caller-owned device buffers:
@@ -210,6 +221,9 @@ int ska_baseline_reg_f64(const double* d_R, const double* d_t, int64_t T, int32_
 #define SKA_BA_CTRL_ACCEPTED 8  /* out: last decision */
 
 #define SKA_BA_FORCE_WIDE 1u    /* flags: run the shared-memory SYRK linearisation even for C == 2 (testing) */
+#define SKA_BA_LOSS_L2 0        /* SkaBaProblem.loss: plain squared pixel error (a zeroed struct) */
+#define SKA_BA_LOSS_HUBER 1
+#define SKA_BA_LOSS_CAUCHY 2
 #define SKA_BA_TENSOR_CORE 2u   /* flags: 5..8 cameras: Schur accumulation on the tensor cores (tcgen05 kind::tf32, three-product split).
                                    Same reduced system to fp32 accuracy; measured SLOWER than the CUDA-core form on B200
                                    (26.3 vs 23.1 ms per 1M x 70 x 8 linearisation, profiles/README.md), hence opt-in */
@@ -239,6 +253,8 @@ typedef struct SkaBaProblem {
                            ska_ba_calib_solve_f64 all-reduce d_red over NVLink peer memory in their prologue and
                            ska_ba_control_f64 / ska_ba_calib_control_f64 do the same for d_red2 - exchange and consumer are ONE
                            kernel, and the caller runs no collective: linearize -> solve -> backsub -> control */
+  int32_t loss;         /* SKA_BA_LOSS_*: read by the linearize and backsub entry points (solve and control ignore it) */
+  double loss_scale;    /* robust scale d in pixels: finite and > 0 unless loss == SKA_BA_LOSS_L2 */
 } SkaBaProblem;
 
 int32_t ska_ba_red_doubles(int32_t C);
@@ -269,8 +285,10 @@ int ska_ba_control_f64(const SkaBaProblem* p, void* stream);
  *   d_delta [C * SKA_BA_CALIB_PARAMS]
  *   d_red   [ska_ba_calib_red_doubles(C)]: upper triangle of Sw (n(n+1)/2, n = 15 C - 6: camera 0 contributes its 9
  *           intrinsics only), then per camera 160 doubles: the row-major upper triangle (153) of sum w row^T row with
- *           row = [B(15) | e | a.dp0] - entries (r,s<=14) Hcc, (r,15) gc, (r,16) bw, (15,15) cost - and, in slot 153,
- *           the count of depth-clamped observations; all sums with raw conf weights
+ *           row = [B(15) | e | a.dp0] - entries (r,s<=14) Hcc, (r,15) gc, (r,16) bw, (15,15) sum w omega s - in slot 153,
+ *           the count of depth-clamped observations, and in slot 154 the robust cost correction sum w (rho(s) - omega s)
+ *           (0 under L2; the data cost is (15,15) + slot 154); all sums with raw conf weights
+ * The robust loss applies as above; depth-clamped observations stay excluded.
  *   d_workspace >= ska_ba_calib_workspace_bytes(C)
  * free_mask: bit (15*c + r) set = parameter r of camera c is optimised (bits 0..5 of camera 0 are ignored).
  * d_prior: nullable [C][18] = theta0(9), rho(9) per camera.

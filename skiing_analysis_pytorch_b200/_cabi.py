@@ -5,7 +5,7 @@ import ctypes as C
 
 import numpy as np
 
-ABI_VERSION = 8
+ABI_VERSION = 9
 MAX_VIEWS = 8
 MAX_BA_VIEWS = 8
 MAX_BONES = 16
@@ -31,6 +31,8 @@ BA_CTRL_COST, BA_CTRL_ACCEPTED = 7, 8
 BA_CTRL_PRIOR_CUR, BA_CTRL_PRIOR_TRIAL = 9, 10  # calibrating BA, written by the solve: intrinsics-prior cost at the current / trial cameras
 BA_FORCE_WIDE = 1
 BA_TENSOR_CORE = 2
+BA_LOSS_L2, BA_LOSS_HUBER, BA_LOSS_CAUCHY = 0, 1, 2
+BA_LOSSES = {"l2": BA_LOSS_L2, "huber": BA_LOSS_HUBER, "cauchy": BA_LOSS_CAUCHY}
 
 ERRORS = {-1: "SKA_EINVAL", -2: "SKA_EUNSUPPORTED", -3: "SKA_EALIGN", -4: "SKA_EWORKSPACE"}
 SKA_EWORKSPACE = -4
@@ -65,6 +67,8 @@ class SkaBaProblem(C.Structure):
         ("ws_bytes", C.c_size_t),
         ("hist_rows", C.c_int64),
         ("peer", C.c_void_p),
+        ("loss", C.c_int32),
+        ("loss_scale", C.c_double),
     ]
 
 

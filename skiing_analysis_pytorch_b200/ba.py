@@ -132,12 +132,22 @@ class BundleAdjuster(LMSequencer):
     group torch.distributed process group when the clip is sharded by frame range over ranks
           (None = the default group when torch.distributed is initialised with world size > 1);
           local_only=True solves this rank's data alone, without any collective
+    loss  "l2" (default: loss.py's squared pixel error), "huber" or "cauchy": a robust M-estimator against gross 2D
+          detector failures, solved by iteratively reweighted Gauss-Newton (include/ska.h, DESIGN.md section 5);
+    loss_scale  its scale in pixels (required, > 0, for "huber" / "cauchy").  `history` and `cost` report the robust cost
     """
 
     def __init__(self, x2d, conf, K, R0, t0, X0, *, layout: str = "TCJ2", mode: str = "full", lam0: float = 1e-3,
                  max_iters: int = 64, group=None, force_wide: bool = False, local_only: bool = False, tensor_core: bool = False,
-                 peer_exchange: bool = True, fuse_exchange: bool = True):
+                 peer_exchange: bool = True, fuse_exchange: bool = True, loss: str = "l2", loss_scale=None):
         self.local_only = bool(local_only)
+        if loss not in _cabi.BA_LOSSES:
+            raise ValueError(f"unknown loss {loss!r}; expected one of {tuple(_cabi.BA_LOSSES)}")
+        if loss != "l2":
+            if loss_scale is None or not np.isfinite(float(loss_scale)) or float(loss_scale) <= 0.0:
+                raise ValueError(f"loss={loss!r} needs a finite loss_scale > 0 (pixels), got {loss_scale!r}")
+            if tensor_core:
+                raise ValueError("tensor_core=True implements the L2 loss only")
         if not (x2d.is_cuda and conf.is_cuda and X0.is_cuda):
             raise RuntimeError("x2d, conf and X0 must be CUDA tensors: this package has no CPU path")
         if x2d.dtype != torch.float32 or conf.dtype != torch.float32:
@@ -209,7 +219,9 @@ class BundleAdjuster(LMSequencer):
             d_red2=self.red2.data_ptr(), d_delta=self.delta.data_ptr(), d_hist=self.hist.data_ptr(),
             d_workspace=self.ws.data_ptr(), ws_bytes=ws, hist_rows=self.max_iters,
             peer=(C.addressof(self.peer.comm) if fuse_exchange and self.peer is not None and self.peer.slot >= 1024 else None),
+            loss=_cabi.BA_LOSSES[loss], loss_scale=(float(loss_scale) if loss != "l2" else 0.0),
         )
+        self.loss = loss
         self.fused_exchange = bool(self.prob.peer)
         self._graph = None
         self.iters_done = 0

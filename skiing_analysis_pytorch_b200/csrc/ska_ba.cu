@@ -64,6 +64,8 @@ struct BaKernelArgs {
   const double* delta;  // [C][6] (backsub)
   float* Xpp;           // [2][N][3] ping-pong
   double* partials;     // [grid][row]
+  int32_t loss;         // SKA_BA_LOSS_* (the kernel's Loss template argument selects the code)
+  float loss_scale;     // robust scale d in pixels (unused by L2)
 };
 
 template <int C>
@@ -96,7 +98,7 @@ __device__ __forceinline__ void load_point(const BaKernelArgs& a, const float* _
 
 // ------------------------------------------------------------------------------------------------
 // linearise, register path (C == 2: one free camera, 56 fp32 accumulators per thread)
-template <int C>
+template <int C, int Loss>
 __global__ void __launch_bounds__(kBaBlock, 2) ba_linearize_reg(const BaKernelArgs a) {
   using L = RedConst<C>;
   static_assert(C == 2, "register path holds the whole reduced system per thread: C == 2 only");
@@ -125,9 +127,17 @@ __global__ void __launch_bounds__(kBaBlock, 2) ba_linearize_reg(const BaKernelAr
       project_lin(s_cam[c], o.X, o.u[c], o.v[c], ol);
       float au[3], av[3];
       point_rows(s_cam[c], ol, au, av);
-      const float cw = o.cw[c];
-      pb_add(pb, cw, au, av, ol.eu, ol.ev);
-      cost = fmaf(cw, fmaf(ol.eu, ol.eu, ol.ev * ol.ev), cost);
+      float cw = o.cw[c];
+      if constexpr (Loss == kLossL2) {  // written out: the robust form below moves this kernel's register allocation
+        pb_add(pb, cw, au, av, ol.eu, ol.ev);
+        cost = fmaf(cw, fmaf(ol.eu, ol.eu, ol.ev * ol.ev), cost);
+      } else {
+        float rho, om;
+        robust_loss<Loss>(fmaf(ol.eu, ol.eu, ol.ev * ol.ev), a.loss_scale, rho, om);
+        cost = fmaf(cw, rho, cost);
+        cw *= om;
+        pb_add(pb, cw, au, av, ol.eu, ol.ev);
+      }
       ncl += ol.clamped ? 1 : 0;
       if (c >= 1) {
         float bu[6], bv[6];
@@ -173,7 +183,7 @@ __global__ void __launch_bounds__(kBaBlock, 2) ba_linearize_reg(const BaKernelAr
 // back-substitution + trial point + trial cost
 constexpr int kBackAcc = 3;  // trial cost, predicted decrease (points), clamped count
 
-template <int C>
+template <int C, int Loss>
 __global__ void __launch_bounds__(kBaBlock, 2) ba_backsub_kernel(const BaKernelArgs a) {
   __shared__ CamF s_cam[C], s_trial[C];
   __shared__ float s_delta[C][6];
@@ -203,7 +213,9 @@ __global__ void __launch_bounds__(kBaBlock, 2) ba_backsub_kernel(const BaKernelA
       project_lin(s_cam[c], o.X, o.u[c], o.v[c], ol);
       float au[3], av[3];
       point_rows(s_cam[c], ol, au, av);
-      const float cw = o.cw[c];
+      float rho, om;  // the linearisation's weight: the same fp32 expression at the same state
+      robust_loss<Loss>(fmaf(ol.eu, ol.eu, ol.ev * ol.ev), a.loss_scale, rho, om);
+      const float cw = o.cw[c] * om;
       pb_add(pb, cw, au, av, ol.eu, ol.ev);
       float lu = ol.eu, lv = ol.ev;
       if (c >= 1) {
@@ -240,7 +252,9 @@ __global__ void __launch_bounds__(kBaBlock, 2) ba_backsub_kernel(const BaKernelA
 #pragma unroll
     for (int c = 0; c < C; ++c) {
       bool cl;
-      tc = fmaf(o.cw[c], project_err2(s_trial[c], Xt, o.u[c], o.v[c], cl), tc);
+      float rho, om;
+      robust_loss<Loss>(project_err2(s_trial[c], Xt, o.u[c], o.v[c], cl), a.loss_scale, rho, om);
+      tc = fmaf(o.cw[c], rho, tc);
       ncl += cl ? 1 : 0;
     }
     acc[0] += tc;
@@ -502,6 +516,8 @@ static int fill_layout(const SkaBaProblem& in, BaKernelArgs& a) {
   a.delta = in.d_delta;
   a.Xpp = in.d_Xpp;
   a.partials = (double*)in.d_workspace;
+  a.loss = in.loss;
+  a.loss_scale = (float)in.loss_scale;
   return SKA_OK;
 }
 
@@ -511,33 +527,49 @@ int launch_reduce(const double* partials, int rows, int ncol, double* out, cudaS
   return ce == cudaSuccess ? SKA_OK : set_error((int)ce, cudaGetErrorString(ce));
 }
 
+template <int Loss>
+static int linearize_reg(const SkaBaProblem& in, const BaKernelArgs& a, cudaStream_t s) {
+  int grid = 1;
+  const int rc = grid_for((const void*)ba_linearize_reg<2, Loss>, a.N, grid);
+  if (rc != SKA_OK) return rc;
+  const size_t need = (size_t)grid * RedConst<2>::size * sizeof(double);
+  if (in.ws_bytes < need) return set_error(SKA_EWORKSPACE, "workspace too small (see ska_ba_workspace_bytes)");
+  ba_linearize_reg<2, Loss><<<grid, kBaBlock, 0, s>>>(a);
+  cudaError_t ce = cudaGetLastError();
+  if (ce != cudaSuccess) return set_error((int)ce, cudaGetErrorString(ce));
+  return launch_reduce(a.partials, grid, RedConst<2>::size, in.d_red, s);
+}
+
 int ba_linearize(const SkaBaProblem& in, cudaStream_t s) {
   if (in.C != 2 || (in.flags & SKA_BA_FORCE_WIDE)) return ba_linearize_wide(in, s);
   BaKernelArgs a;
   fill_layout(in, a);
-  {
-    int grid = 1;
-    const int rc = grid_for((const void*)ba_linearize_reg<2>, a.N, grid);
-    if (rc != SKA_OK) return rc;
-    const size_t need = (size_t)grid * RedConst<2>::size * sizeof(double);
-    if (in.ws_bytes < need) return set_error(SKA_EWORKSPACE, "workspace too small (see ska_ba_workspace_bytes)");
-    ba_linearize_reg<2><<<grid, kBaBlock, 0, s>>>(a);
-    cudaError_t ce = cudaGetLastError();
-    if (ce != cudaSuccess) return set_error((int)ce, cudaGetErrorString(ce));
-    return launch_reduce(a.partials, grid, RedConst<2>::size, in.d_red, s);
+  switch (in.loss) {
+    case SKA_BA_LOSS_HUBER: return linearize_reg<kLossHuber>(in, a, s);
+    case SKA_BA_LOSS_CAUCHY: return linearize_reg<kLossCauchy>(in, a, s);
+    default: return linearize_reg<kLossL2>(in, a, s);
   }
+}
+
+template <int C, int Loss>
+static int backsub_cl(const SkaBaProblem& in, const BaKernelArgs& a, cudaStream_t s) {
+  int grid = 1;
+  const int rc = grid_for((const void*)ba_backsub_kernel<C, Loss>, a.N, grid);
+  if (rc != SKA_OK) return rc;
+  if (in.ws_bytes < (size_t)grid * kBackAcc * sizeof(double)) return set_error(SKA_EWORKSPACE, "workspace too small (see ska_ba_workspace_bytes)");
+  ba_backsub_kernel<C, Loss><<<grid, kBaBlock, 0, s>>>(a);
+  cudaError_t ce = cudaGetLastError();
+  if (ce != cudaSuccess) return set_error((int)ce, cudaGetErrorString(ce));
+  return launch_reduce(a.partials, grid, kBackAcc, in.d_red2, s);
 }
 
 template <int C>
 static int backsub_c(const SkaBaProblem& in, const BaKernelArgs& a, cudaStream_t s) {
-  int grid = 1;
-  const int rc = grid_for((const void*)ba_backsub_kernel<C>, a.N, grid);
-  if (rc != SKA_OK) return rc;
-  if (in.ws_bytes < (size_t)grid * kBackAcc * sizeof(double)) return set_error(SKA_EWORKSPACE, "workspace too small (see ska_ba_workspace_bytes)");
-  ba_backsub_kernel<C><<<grid, kBaBlock, 0, s>>>(a);
-  cudaError_t ce = cudaGetLastError();
-  if (ce != cudaSuccess) return set_error((int)ce, cudaGetErrorString(ce));
-  return launch_reduce(a.partials, grid, kBackAcc, in.d_red2, s);
+  switch (in.loss) {
+    case SKA_BA_LOSS_HUBER: return backsub_cl<C, kLossHuber>(in, a, s);
+    case SKA_BA_LOSS_CAUCHY: return backsub_cl<C, kLossCauchy>(in, a, s);
+    default: return backsub_cl<C, kLossL2>(in, a, s);
+  }
 }
 
 int ba_backsub(const SkaBaProblem& in, cudaStream_t s) {

@@ -61,6 +61,31 @@ __device__ __forceinline__ float ba_rcp(float z) {
   return fmaf(r, fmaf(-z, r, 1.0f), r);
 }
 
+// Robust loss of one observation's squared pixel error s = e_u^2 + e_v^2 (tests/oracle_robust.py, DESIGN.md section 5):
+//   l2      rho = s                                  omega = 1
+//   huber   rho = s (s <= d^2), 2 d sqrt(s) - d^2    omega = 1 (s <= d^2), d / sqrt(s)
+//   cauchy  rho = d^2 ln(1 + s / d^2)                omega = 1 / (1 + s / d^2)
+// The kernels weight the observation by conf * omega in every sum of the step (iteratively reweighted Gauss-Newton,
+// omega not differentiated) and add conf * rho to the cost.  Huber's inlier branch is the L2 expression itself, so a
+// solve whose every residual lies inside d is bit-identical to L2.  `d` is the scale in pixels (> 0).
+enum : int { kLossL2 = 0, kLossHuber = 1, kLossCauchy = 2 };  // SKA_BA_LOSS_* (include/ska.h)
+
+template <int Loss>
+__device__ __forceinline__ void robust_loss(float s, float d, float& rho, float& omega) {
+  if constexpr (Loss == kLossHuber) {
+    const bool in = s <= d * d;
+    omega = in ? 1.0f : d * rsqrtf(s);
+    rho = in ? s : fmaf(2.0f * s, omega, -(d * d));  // 2 s d / sqrt(s) = 2 d sqrt(s)
+  } else if constexpr (Loss == kLossCauchy) {
+    const float q = s * ba_rcp(d * d);
+    omega = ba_rcp(1.0f + q);
+    rho = (d * d) * log1pf(q);
+  } else {
+    rho = s;
+    omega = 1.0f;
+  }
+}
+
 // One observation: residual e, Jacobian rows of (u,v) w.r.t. X_c (ju, jv) and p = R X.
 struct ObsLin {
   float eu, ev;

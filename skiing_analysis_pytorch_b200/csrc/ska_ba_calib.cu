@@ -14,7 +14,8 @@
 //   [0, n(n+1)/2)        upper triangle of Sw = sum_points Y^T Y,  Y = L^-1 W   (L L^T = damped 3x3 point block)
 //   then per camera c    160 doubles: the upper triangle (153) of  sum_obs w row^T row  with the 17-entry row
 //                        [B (15) | e | a.dp0]: entries (r,s<=14) = Hcc, (r,15) = gc, (r,16) = bw, (15,15) = cost;
-//                        slot 153 = number of depth-clamped observations
+//                        slot 153 = number of depth-clamped observations; slot 154 = the robust cost correction
+//                        sum w (rho(s) - omega s), so that (15,15) + slot 154 = sum w rho(s) (0 under L2)
 // all sums with the raw confidences; the fp64 solve / control kernels scale by 1/(sum conf + 1e-6) once.
 //
 // ba_calib_linearize_kernel<C>: a warp owns 32 points per tile.
@@ -80,6 +81,8 @@ struct CalibArgs {
   const double* delta;  // [C][15]
   float* Xpp;
   double* partials;
+  int32_t loss;       // SKA_BA_LOSS_* (the kernel's Loss template argument selects the code)
+  float loss_scale;   // robust scale d in pixels (unused by L2)
 };
 
 __device__ __forceinline__ void load_cam_calib(const double* __restrict__ s, CamC& c) {
@@ -93,30 +96,33 @@ __device__ __forceinline__ void load_cam_calib(const double* __restrict__ s, Cam
 
 // product Q of the per-camera block, resolved at compile time
 template <int Q>
-__device__ __forceinline__ float calib_prod(const float (&su)[kCalibRow], const float (&sv)[kCalibRow], const ObsCalib& o, float clampv) {
+__device__ __forceinline__ float calib_prod(const float (&su)[kCalibRow], const float (&sv)[kCalibRow], const ObsCalib& o, float clampv,
+                                            float robustv) {
   if constexpr (Q < kCalibTri) {
     constexpr int r = calib_tri_row(Q), s = calib_tri_col(Q);
     return fmaf(su[r], o.bu[s], sv[r] * o.bv[s]);
   } else if constexpr (Q == kCalibClampSlot) {
     return clampv;
+  } else if constexpr (Q == kCalibRobustSlot) {
+    return robustv;
   } else {
     return 0.0f;
   }
 }
 template <int B, int... I>
 __device__ __forceinline__ void calib_fill(float (&v)[32], const float (&su)[kCalibRow], const float (&sv)[kCalibRow], const ObsCalib& o,
-                                           float clampv, std::integer_sequence<int, I...>) {
-  ((v[I] = calib_prod<32 * B + I>(su, sv, o, clampv)), ...);
+                                           float clampv, float robustv, std::integer_sequence<int, I...>) {
+  ((v[I] = calib_prod<32 * B + I>(su, sv, o, clampv, robustv)), ...);
 }
 template <int B>
 __device__ __forceinline__ float calib_batch(const float (&su)[kCalibRow], const float (&sv)[kCalibRow], const ObsCalib& o, float clampv,
-                                             int lane) {
+                                             float robustv, int lane) {
   float v[32];
-  calib_fill<B>(v, su, sv, o, clampv, std::make_integer_sequence<int, 32>{});
+  calib_fill<B>(v, su, sv, o, clampv, robustv, std::make_integer_sequence<int, 32>{});
   return transpose_reduce32(v, lane);
 }
 
-template <int C>
+template <int C, int Loss>
 __global__ void __launch_bounds__(32 * Calib<C>::W, 1) ba_calib_linearize_kernel(const CalibArgs a) {
   using L = Calib<C>;
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -183,11 +189,20 @@ __global__ void __launch_bounds__(32 * Calib<C>::W, 1) ba_calib_linearize_kernel
     }
     PointBlock pb;
     pb_zero(pb);
+    float rcorr[C];  // cw (rho - omega s): slot 154
 #pragma unroll
     for (int c = 0; c < C; ++c) {
       ObsCalib o;
       calib_obs(s_cam[c], Xp, u[c], v[c], o);
       cw[c] = o.clamped ? 0.f : cw[c];  // a depth-clamped observation is excluded (ska_ba_calib.cuh)
+      rcorr[c] = 0.f;
+      if constexpr (Loss != kLossL2) {
+        const float s2 = fmaf(o.bu[15], o.bu[15], o.bv[15] * o.bv[15]);
+        float rho, om;
+        robust_loss<Loss>(s2, a.loss_scale, rho, om);
+        rcorr[c] = cw[c] * fmaf(-om, s2, rho);
+        cw[c] *= om;  // pass B re-linearises the same state: it uses this weight
+      }
       pb_add(pb, cw[c], o.au, o.av, o.bu[15], o.bv[15]);
     }
     const Chol3 f = chol3_damped(pb, lam);
@@ -226,11 +241,11 @@ __global__ void __launch_bounds__(32 * Calib<C>::W, 1) ba_calib_linearize_kernel
         yt[2] = y2;
       }
       const float clampv = (valid && o.clamped) ? 1.f : 0.f;
-      accH[c][0] += calib_batch<0>(su, sv, o, clampv, lane);
-      accH[c][1] += calib_batch<1>(su, sv, o, clampv, lane);
-      accH[c][2] += calib_batch<2>(su, sv, o, clampv, lane);
-      accH[c][3] += calib_batch<3>(su, sv, o, clampv, lane);
-      accH[c][4] += calib_batch<4>(su, sv, o, clampv, lane);
+      accH[c][0] += calib_batch<0>(su, sv, o, clampv, rcorr[c], lane);
+      accH[c][1] += calib_batch<1>(su, sv, o, clampv, rcorr[c], lane);
+      accH[c][2] += calib_batch<2>(su, sv, o, clampv, rcorr[c], lane);
+      accH[c][3] += calib_batch<3>(su, sv, o, clampv, rcorr[c], lane);
+      accH[c][4] += calib_batch<4>(su, sv, o, clampv, rcorr[c], lane);
     }
     __syncwarp();
     // ---------------------------------------------------------------- phase 2: Sw block (pa, pb_)
@@ -297,7 +312,7 @@ __global__ void __launch_bounds__(32 * Calib<C>::W, 1) ba_calib_linearize_kernel
 // back-substitution + trial point + trial cost (thread per point)
 constexpr int kCalibBackAcc = 3;  // trial cost, predicted decrease (points), clamped count
 
-template <int C>
+template <int C, int Loss>
 __global__ void __launch_bounds__(kBaBlock, 2) ba_calib_backsub_kernel(const CalibArgs a) {
   __shared__ CamC s_cam[C], s_trial[C];
   __shared__ float s_delta[C][kCalibP];
@@ -336,7 +351,12 @@ __global__ void __launch_bounds__(kBaBlock, 2) ba_calib_backsub_kernel(const Cal
     for (int c = 0; c < C; ++c) {
       ObsCalib o;
       calib_obs(s_cam[c], Xp, u[c], v[c], o);
-      const float w = o.clamped ? 0.f : cw[c];  // excluded observation
+      float w = o.clamped ? 0.f : cw[c];  // excluded observation
+      if constexpr (Loss != kLossL2) {  // the linearisation's weight: the same fp32 expression at the same state
+        float rho, om;
+        robust_loss<Loss>(fmaf(o.bu[15], o.bu[15], o.bv[15] * o.bv[15]), a.loss_scale, rho, om);
+        w *= om;
+      }
       pb_add(pb, w, o.au, o.av, o.bu[15], o.bv[15]);
       float lu = o.bu[15], lv = o.bv[15];
 #pragma unroll
@@ -368,7 +388,9 @@ __global__ void __launch_bounds__(kBaBlock, 2) ba_calib_backsub_kernel(const Cal
 #pragma unroll
     for (int c = 0; c < C; ++c) {
       bool cl;
-      tc = fmaf(cw[c], calib_err2(s_trial[c], Xt, u[c], v[c], cl), tc);
+      float rho, om;
+      robust_loss<Loss>(calib_err2(s_trial[c], Xt, u[c], v[c], cl), a.loss_scale, rho, om);
+      tc = fmaf(cw[c], rho, tc);
       ncl += cl ? 1 : 0;
     }
     acc[0] += tc;
@@ -517,6 +539,7 @@ __global__ void __launch_bounds__(32) ba_calib_control_kernel(int C, const doubl
     double data = 0.0, ncl = 0.0;
     for (int c = 0; c < C; ++c) {
       data += red[L.oCam + kCalibCamBlock * c + calib_tri(15, 15)];
+      data += red[L.oCam + kCalibCamBlock * c + kCalibRobustSlot];  // robust cost correction; +0.0 under L2
       ncl += red[L.oCam + kCalibCamBlock * c + kCalibClampSlot];
     }
     const double F = s * data + ctrl[kCtrlPriorCur], Ft = s * red2[0] + ctrl[kCtrlPriorTrial];
@@ -582,6 +605,8 @@ static void fill_args(const SkaBaProblem& in, CalibArgs& a) {
   a.delta = in.d_delta;
   a.Xpp = in.d_Xpp;
   a.partials = (double*)in.d_workspace;
+  a.loss = in.loss;
+  a.loss_scale = (float)in.loss_scale;
 }
 
 int ba_calib_red_size(int C) { return CalibLayout(C).size; }
@@ -590,12 +615,12 @@ static int unsupported_c() {
   return set_error(SKA_EUNSUPPORTED, "calibrating BA (free intrinsics / distortion) is built for C == 2 cameras (BASELINE config 3)");
 }
 
-int ba_calib_linearize(const SkaBaProblem& in, cudaStream_t s) {
-  if (in.C != 2) return unsupported_c();
+template <int Loss>
+static int calib_linearize(const SkaBaProblem& in, cudaStream_t s) {
   using L = Calib<2>;
   CalibArgs a;
   fill_args(in, a);
-  auto kern = ba_calib_linearize_kernel<2>;
+  auto kern = ba_calib_linearize_kernel<2, Loss>;
   static bool attr_set[64] = {};
   int dev = 0, sms = 0;
   cudaError_t ce = cudaGetDevice(&dev);
@@ -622,14 +647,23 @@ int ba_calib_linearize(const SkaBaProblem& in, cudaStream_t s) {
   return launch_reduce(a.partials, (int)grid, L::size, in.d_red, s);
 }
 
-int ba_calib_backsub(const SkaBaProblem& in, cudaStream_t s) {
+int ba_calib_linearize(const SkaBaProblem& in, cudaStream_t s) {
   if (in.C != 2) return unsupported_c();
+  switch (in.loss) {
+    case SKA_BA_LOSS_HUBER: return calib_linearize<kLossHuber>(in, s);
+    case SKA_BA_LOSS_CAUCHY: return calib_linearize<kLossCauchy>(in, s);
+    default: return calib_linearize<kLossL2>(in, s);
+  }
+}
+
+template <int Loss>
+static int calib_backsub(const SkaBaProblem& in, cudaStream_t s) {
   CalibArgs a;
   fill_args(in, a);
   int dev = 0, sms = 0, per_sm = 0;
   cudaError_t ce = cudaGetDevice(&dev);
   if (ce == cudaSuccess) ce = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  if (ce == cudaSuccess) ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ba_calib_backsub_kernel<2>, kBaBlock, 0);
+  if (ce == cudaSuccess) ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ba_calib_backsub_kernel<2, Loss>, kBaBlock, 0);
   if (ce != cudaSuccess) return set_error((int)ce, cudaGetErrorString(ce));
   if (per_sm < 1) per_sm = 1;
   int64_t grid = (int64_t)sms * per_sm;
@@ -637,10 +671,19 @@ int ba_calib_backsub(const SkaBaProblem& in, cudaStream_t s) {
   if (grid > need) grid = need;
   if (grid < 1) grid = 1;
   if (in.ws_bytes < (size_t)grid * kCalibBackAcc * sizeof(double)) return set_error(SKA_EWORKSPACE, "workspace too small (see ska_ba_calib_workspace_bytes)");
-  ba_calib_backsub_kernel<2><<<(unsigned)grid, kBaBlock, 0, s>>>(a);
+  ba_calib_backsub_kernel<2, Loss><<<(unsigned)grid, kBaBlock, 0, s>>>(a);
   ce = cudaGetLastError();
   if (ce != cudaSuccess) return set_error((int)ce, cudaGetErrorString(ce));
   return launch_reduce(a.partials, (int)grid, kCalibBackAcc, in.d_red2, s);
+}
+
+int ba_calib_backsub(const SkaBaProblem& in, cudaStream_t s) {
+  if (in.C != 2) return unsupported_c();
+  switch (in.loss) {
+    case SKA_BA_LOSS_HUBER: return calib_backsub<kLossHuber>(in, s);
+    case SKA_BA_LOSS_CAUCHY: return calib_backsub<kLossCauchy>(in, s);
+    default: return calib_backsub<kLossL2>(in, s);
+  }
 }
 
 static int calib_peer_of(const SkaPeerComm* c, int payload, PeerDev& pd) {

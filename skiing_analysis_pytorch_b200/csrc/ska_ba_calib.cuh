@@ -31,6 +31,7 @@ constexpr int kCalibNI = 9;          // intrinsic parameters theta = fx fy cx cy
 constexpr int kCalibRow = 17;        // per-observation row [B (15) | e | a.dp0]
 constexpr int kCalibTri = 153;       // upper triangle of the 17 x 17 per-camera matrix sum w row^T row
 constexpr int kCalibClampSlot = 153; // per-camera count of depth-clamped observations
+constexpr int kCalibRobustSlot = 154; // per-camera robust cost correction sum w (rho(s) - omega s); 0 under L2
 constexpr int kCalibCamBlock = 160;  // padded per-camera block of the packed reduced system (5 x 32)
 constexpr float kCalibZMin = 1e-6f;
 

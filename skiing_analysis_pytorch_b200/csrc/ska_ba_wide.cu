@@ -38,6 +38,8 @@ struct BaKernelArgsW {
   const double* ctrl;
   const float* Xpp;
   double* partials;
+  int32_t loss;       // SKA_BA_LOSS_* (the kernel's Loss template argument selects the code)
+  float loss_scale;   // robust scale d in pixels (unused by L2)
 };
 
 #ifndef SKA_BA_WIDE_WARPS
@@ -60,7 +62,7 @@ struct Wide {
   static constexpr size_t smem = (size_t)W * warp_floats * sizeof(float) + (size_t)size * sizeof(double) + C * sizeof(CamF);
 };
 
-template <int C>
+template <int C, int Loss>
 __global__ void __launch_bounds__(32 * Wide<C>::W, 1) ba_linearize_wide_kernel(const BaKernelArgsW a) {
   using L = Wide<C>;
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -134,8 +136,11 @@ __global__ void __launch_bounds__(32 * Wide<C>::W, 1) ba_linearize_wide_kernel(c
       project_lin(s_cam[c], Xp, u[c], v[c], ol);
       float au[3], av[3];
       point_rows(s_cam[c], ol, au, av);
+      float rho, om;
+      robust_loss<Loss>(fmaf(ol.eu, ol.eu, ol.ev * ol.ev), a.loss_scale, rho, om);
+      cost = fmaf(cw[c], rho, cost);
+      cw[c] *= om;  // pass B below re-projects the same state: it uses this weight
       pb_add(pb, cw[c], au, av, ol.eu, ol.ev);
-      cost = fmaf(cw[c], fmaf(ol.eu, ol.eu, ol.ev * ol.ev), cost);
       nclamp += (valid && ol.clamped) ? 1.f : 0.f;
     }
     const Chol3 f = chol3_damped(pb, lam);
@@ -642,10 +647,10 @@ static int launch_tc(const SkaBaProblem& in, BaKernelArgsW& a, cudaStream_t s) {
   return launch_reduce(a.partials, (int)grid, L::size, in.d_red, s);
 }
 
-template <int C>
+template <int C, int Loss>
 static int launch_wide(const SkaBaProblem& in, BaKernelArgsW& a, cudaStream_t s) {
   using L = Wide<C>;
-  auto kern = ba_linearize_wide_kernel<C>;
+  auto kern = ba_linearize_wide_kernel<C, Loss>;
   static bool attr_set[64] = {};
   int dev = 0, sms = 0;
   cudaError_t ce = cudaGetDevice(&dev);
@@ -672,6 +677,15 @@ static int launch_wide(const SkaBaProblem& in, BaKernelArgsW& a, cudaStream_t s)
   return launch_reduce(a.partials, (int)grid, L::size, in.d_red, s);
 }
 
+template <int C>
+static int launch_wide(const SkaBaProblem& in, BaKernelArgsW& a, cudaStream_t s) {
+  switch (in.loss) {
+    case SKA_BA_LOSS_HUBER: return launch_wide<C, kLossHuber>(in, a, s);
+    case SKA_BA_LOSS_CAUCHY: return launch_wide<C, kLossCauchy>(in, a, s);
+    default: return launch_wide<C, kLossL2>(in, a, s);
+  }
+}
+
 int ba_linearize_wide(const SkaBaProblem& in, cudaStream_t s) {
   BaKernelArgsW a;
   a.N = in.T * (int64_t)in.J;
@@ -693,8 +707,11 @@ int ba_linearize_wide(const SkaBaProblem& in, cudaStream_t s) {
   a.ctrl = in.d_ctrl;
   a.Xpp = in.d_Xpp;
   a.partials = (double*)in.d_workspace;
+  a.loss = in.loss;
+  a.loss_scale = (float)in.loss_scale;
 #ifndef SKA_BA_NO_TC
   if (in.C >= 5 && (in.flags & SKA_BA_TENSOR_CORE) && !(in.flags & SKA_BA_FORCE_WIDE)) {  // opt-in: measured slower than the CUDA-core form below
+    if (in.loss != SKA_BA_LOSS_L2) return set_error(SKA_EUNSUPPORTED, "the tensor-core Schur form implements the L2 loss only");
     switch (in.C) {
       case 5: return launch_tc<5>(in, a, s);
       case 6: return launch_tc<6>(in, a, s);

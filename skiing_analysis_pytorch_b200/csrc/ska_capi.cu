@@ -1,5 +1,6 @@
 // ska_capi.cu - the extern "C" boundary of libska.so: argument validation and dispatch only.
 #include <cuda_runtime.h>
+#include <float.h>
 #include <stdio.h>
 #include <string.h>
 
@@ -241,6 +242,13 @@ static int check_problem(const SkaBaProblem* p, bool need_points) {
     if (p->d_workspace == nullptr) return set_error(SKA_EINVAL, "d_workspace must not be NULL");
     if (reinterpret_cast<uintptr_t>(p->d_x2d) % 8 != 0) return set_error(SKA_EALIGN, "d_x2d must be 8-byte aligned");
     if (reinterpret_cast<uintptr_t>(p->d_workspace) % 16 != 0) return set_error(SKA_EALIGN, "d_workspace must be 16-byte aligned");
+    // the loss is read by the per-observation kernels only (solve / control ignore it); they hold d and d^2 in fp32
+    if (p->loss != SKA_BA_LOSS_L2 && p->loss != SKA_BA_LOSS_HUBER && p->loss != SKA_BA_LOSS_CAUCHY) return set_error(SKA_EINVAL, "unknown loss");
+    if (p->loss != SKA_BA_LOSS_L2) {
+      const float d = (float)p->loss_scale;
+      if (!(isfinite(p->loss_scale) && p->loss_scale > 0.0 && isfinite(d * d) && d * d >= FLT_MIN))
+        return set_error(SKA_EINVAL, "a robust loss needs a finite loss_scale > 0 whose square is a normal fp32 number");
+    }
   }
   return SKA_OK;
 }

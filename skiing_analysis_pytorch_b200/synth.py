@@ -118,6 +118,32 @@ def make_clip(rig_name: str, T: int, J: int, seed: int = 0, noise_px: float = 1.
     return Clip(X=X, R=R, t=t, K=K, x_vm=x, conf_vm=conf)
 
 
+def inject_outliers(x2d: np.ndarray, J: int, frac: float, seed: int = 0) -> np.ndarray:
+    """Corrupt a fraction `frac` of the observations of x2d (..., J, 2) IN PLACE, the way monocular 2D detectors fail
+    (swapped limbs, invented positions of occluded joints), and return the (..., J) bool mask of corrupted ones.
+    Half of them take another joint's observation of the same frame and view (a limb swap); the other half move by a
+    uniform 50-300 px in a uniform direction.  Confidences are not touched: they do not flag the outliers."""
+    if x2d.shape[-2:] != (J, 2):
+        raise ValueError(f"x2d must end in ({J}, 2), got {x2d.shape}")
+    rng = np.random.default_rng(seed)
+    flat = x2d.reshape(-1, J, 2)
+    n = flat.shape[0] * J
+    k = int(round(frac * n))
+    pick = rng.choice(n, size=k, replace=False)
+    row, j = pick // J, pick % J
+    orig = flat.copy()
+    half = k // 2
+    if J > 1:
+        other = (j[:half] + rng.integers(1, J, half)) % J
+        flat[row[:half], j[:half]] = orig[row[:half], other]
+    r = rng.uniform(50.0, 300.0, k - half)
+    phi = rng.uniform(0.0, 2 * np.pi, k - half)
+    flat[row[half:], j[half:]] = orig[row[half:], j[half:]] + np.stack([r * np.cos(phi), r * np.sin(phi)], -1).astype(flat.dtype)
+    mask = np.zeros(n, bool)
+    mask[pick] = True
+    return mask.reshape(x2d.shape[:-1])
+
+
 def so3_exp(w):
     w = np.asarray(w, float)
     th = np.linalg.norm(w)
