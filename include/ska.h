@@ -334,7 +334,23 @@ int ska_ba_calib_control_f64(const SkaBaProblem* p, void* stream);
  *   repeat: [halo exchange of p] cg(MATVEC) -> [all-reduce DOT] -> cg(ALPHA) -> cg(UPDATE) -> [all-reduce DOT] -> cg(BETA) -> cg(DIR)
  *           (a fixed number of times: once converged every kernel returns at once - no host round trip)
  *   ska_ba_reg_apply_f64 -> [halo exchange of the trial X / cameras] -> ska_ba_reg_cost_f64(p, 1) -> [all-reduce d_sums[1]]
- *   -> ska_ba_reg_finish_cost_f64(p, 1) -> ska_ba_reg_control_f64 */
+ *   -> ska_ba_reg_finish_cost_f64(p, 1) -> ska_ba_reg_control_f64
+ *
+ * Robust loss (ska_ba_reg_{cost,linearize,cg}_robust_f64; `loss` = SKA_BA_LOSS_*, `loss_scale` = d in pixels): rho and omega
+ * as in the Schur-LM section above, on the REPROJECTION group only.  Its term becomes c_r sum conf rho(s), s = e_u^2 + e_v^2
+ * (c_r still from the raw sum of conf); bone length, pose temporal, smoothness and baseline stay squared.  The step is
+ * iteratively reweighted Gauss-Newton: every reprojection contribution to g, D, the matrix-vector product and the frame
+ * preconditioner uses the weight c_r conf omega(s), omega at the current point and not differentiated, so g is still half
+ * the gradient of F and the predicted decrease, the gain ratio and the accept rule keep their meaning.  Depth-clamped
+ * observations keep their residual and are weighted by omega of it.  d_sums' reprojection column, the history's `reproj`
+ * and `cost` are the robust values; the clamp count is unchanged.  Huber computes an inlier with the L2 expressions: a
+ * solve with every residual inside d is bit-identical to L2.
+ *   - The loss and scale must be the same for every call of a trial (the kernels recompute omega from the observations
+ *     instead of storing it, so the linearisation and the CG operators agree bit for bit only then).
+ *   - cg ops that read no observations (INIT, ALPHA, BETA, DIR, and BEGIN / UPDATE with free_mask == 0) ignore it.
+ *   - An unknown loss, or for a robust loss a scale that is not finite and > 0 with d^2 a normal fp64 number, returns
+ *     SKA_EINVAL before any CUDA call.
+ * ska_ba_reg_cost_f64 / _linearize_f64 / _cg_f64 are the robust entry points with SKA_BA_LOSS_L2. */
 #define SKA_BA_REG_NVEC 7
 #define SKA_BA_REG_SUMS 40
 #define SKA_BA_REG_SC_DOUBLES 64
@@ -387,6 +403,9 @@ int ska_ba_reg_linearize_f64(const SkaBaRegProblem* p, void* stream);
 int ska_ba_reg_cg_f64(const SkaBaRegProblem* p, int32_t op, void* stream);
 int ska_ba_reg_apply_f64(const SkaBaRegProblem* p, void* stream);
 int ska_ba_reg_control_f64(const SkaBaRegProblem* p, void* stream);
+int ska_ba_reg_cost_robust_f64(const SkaBaRegProblem* p, int32_t which, int32_t loss, double loss_scale, void* stream);
+int ska_ba_reg_linearize_robust_f64(const SkaBaRegProblem* p, int32_t loss, double loss_scale, void* stream);
+int ska_ba_reg_cg_robust_f64(const SkaBaRegProblem* p, int32_t op, int32_t loss, double loss_scale, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * The exchange step of the sharded solvers over NVLink peer memory (SURVEY row e: the NCCL all-reduce of the packed

@@ -34,6 +34,18 @@ BA_TENSOR_CORE = 2
 BA_LOSS_L2, BA_LOSS_HUBER, BA_LOSS_CAUCHY = 0, 1, 2
 BA_LOSSES = {"l2": BA_LOSS_L2, "huber": BA_LOSS_HUBER, "cauchy": BA_LOSS_CAUCHY}
 
+
+def check_loss(loss, loss_scale):
+    """A solver's `loss` / `loss_scale` arguments as the C ABI takes them: (SKA_BA_LOSS_* value, scale in pixels, 0.0 for
+    "l2"), or ValueError."""
+    if loss not in BA_LOSSES:
+        raise ValueError(f"unknown loss {loss!r}; expected one of {tuple(BA_LOSSES)}")
+    if loss == "l2":
+        return BA_LOSS_L2, 0.0
+    if loss_scale is None or not np.isfinite(float(loss_scale)) or float(loss_scale) <= 0.0:
+        raise ValueError(f"loss={loss!r} needs a finite loss_scale > 0 (pixels), got {loss_scale!r}")
+    return BA_LOSSES[loss], float(loss_scale)
+
 ERRORS = {-1: "SKA_EINVAL", -2: "SKA_EUNSUPPORTED", -3: "SKA_EALIGN", -4: "SKA_EWORKSPACE"}
 SKA_EWORKSPACE = -4
 

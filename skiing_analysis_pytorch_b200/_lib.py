@@ -72,6 +72,9 @@ _SIGS = {
     "ska_ba_reg_cg_f64": (C.c_int, [C.POINTER(_cabi.SkaBaRegProblem), C.c_int32, _vp]),
     "ska_ba_reg_apply_f64": (C.c_int, [C.POINTER(_cabi.SkaBaRegProblem), _vp]),
     "ska_ba_reg_control_f64": (C.c_int, [C.POINTER(_cabi.SkaBaRegProblem), _vp]),
+    "ska_ba_reg_cost_robust_f64": (C.c_int, [C.POINTER(_cabi.SkaBaRegProblem), C.c_int32, C.c_int32, C.c_double, _vp]),
+    "ska_ba_reg_linearize_robust_f64": (C.c_int, [C.POINTER(_cabi.SkaBaRegProblem), C.c_int32, C.c_double, _vp]),
+    "ska_ba_reg_cg_robust_f64": (C.c_int, [C.POINTER(_cabi.SkaBaRegProblem), C.c_int32, C.c_int32, C.c_double, _vp]),
     "ska_peer_region_bytes": (C.c_size_t, [C.c_int32, C.c_int32]),
     "ska_peer_alloc": (C.c_int, [C.c_size_t, C.POINTER(C.c_void_p)]),
     "ska_peer_free": (C.c_int, [_vp]),

@@ -141,13 +141,9 @@ class BundleAdjuster(LMSequencer):
                  max_iters: int = 64, group=None, force_wide: bool = False, local_only: bool = False, tensor_core: bool = False,
                  peer_exchange: bool = True, fuse_exchange: bool = True, loss: str = "l2", loss_scale=None):
         self.local_only = bool(local_only)
-        if loss not in _cabi.BA_LOSSES:
-            raise ValueError(f"unknown loss {loss!r}; expected one of {tuple(_cabi.BA_LOSSES)}")
-        if loss != "l2":
-            if loss_scale is None or not np.isfinite(float(loss_scale)) or float(loss_scale) <= 0.0:
-                raise ValueError(f"loss={loss!r} needs a finite loss_scale > 0 (pixels), got {loss_scale!r}")
-            if tensor_core:
-                raise ValueError("tensor_core=True implements the L2 loss only")
+        loss_id, loss_scale = _cabi.check_loss(loss, loss_scale)
+        if loss != "l2" and tensor_core:
+            raise ValueError("tensor_core=True implements the L2 loss only")
         if not (x2d.is_cuda and conf.is_cuda and X0.is_cuda):
             raise RuntimeError("x2d, conf and X0 must be CUDA tensors: this package has no CPU path")
         if x2d.dtype != torch.float32 or conf.dtype != torch.float32:
@@ -219,7 +215,7 @@ class BundleAdjuster(LMSequencer):
             d_red2=self.red2.data_ptr(), d_delta=self.delta.data_ptr(), d_hist=self.hist.data_ptr(),
             d_workspace=self.ws.data_ptr(), ws_bytes=ws, hist_rows=self.max_iters,
             peer=(C.addressof(self.peer.comm) if fuse_exchange and self.peer is not None and self.peer.slot >= 1024 else None),
-            loss=_cabi.BA_LOSSES[loss], loss_scale=(float(loss_scale) if loss != "l2" else 0.0),
+            loss=loss_id, loss_scale=loss_scale,
         )
         self.loss = loss
         self.fused_exchange = bool(self.prob.peer)
@@ -717,7 +713,8 @@ def run_local_ba_first_order(K_torch, R_init_torch, t_init_torch, X3d_init_torch
 
 
 def run_local_ba(K_torch, R_init_torch, t_init_torch, X3d_init_torch, x2d_torch, conf2d_torch, num_iters=200, lr=1e-3,
-                 device="cuda", mode="pose_only", optimizer="adam", weights=None, graph=True, fused=True, static_rig_tol=1e-6):
+                 device="cuda", mode="pose_only", optimizer="adam", weights=None, graph=True, fused=True, static_rig_tol=1e-6,
+                 loss="l2", loss_scale=None):
     """The optimiser the reference calls but never defines (vggt/multi_view_process.py:553-564;
     argument shapes :546-551).  Returns (R_opt (T,C,3,3), t_opt (T,C,3), X_opt (T,J,3), history).
 
@@ -734,7 +731,13 @@ def run_local_ba(K_torch, R_init_torch, t_init_torch, X3d_init_torch, x2d_torch,
     only if they ARE one rig: they may differ from their mean (chordal mean rotation, mean translation) by at most
     `static_rig_tol` (radians / translation units), otherwise ValueError - averaging a moving rig silently would pull the
     points towards cameras they were not seen by.  mode="pose_only" returns the input cameras untouched (only the
-    points move); `lr` is used as the initial damping lambda0; `num_iters` is capped at 64 trials (LM converges in ~10)."""
+    points move); `lr` is used as the initial damping lambda0; `num_iters` is capped at 64 trials (LM converges in ~10).
+
+    loss="huber" | "cauchy" with loss_scale (pixels): a robust loss on the reprojection term against gross 2D detector
+    failures, for optimizer="lm" and "lm_rig" (include/ska.h); the default "l2" is loss.py's squared error."""
+    _cabi.check_loss(loss, loss_scale)
+    if optimizer == "adam" and loss != "l2":
+        raise ValueError(f"loss={loss!r} is implemented by optimizer='lm' and 'lm_rig'; optimizer='adam' minimises the L2 loss only")
     if optimizer == "adam":
         return run_local_ba_first_order(K_torch, R_init_torch, t_init_torch, X3d_init_torch, x2d_torch, conf2d_torch, num_iters, lr,
                                         device, mode, weights, graph, fused)
@@ -744,7 +747,7 @@ def run_local_ba(K_torch, R_init_torch, t_init_torch, X3d_init_torch, x2d_torch,
         if mode not in MODES:
             raise ValueError(f"unknown mode {mode!r}; expected one of {MODES}")
         return ba_reg.run_local_ba_lm(K_torch, R_init_torch, t_init_torch, X3d_init_torch, x2d_torch, conf2d_torch, num_iters, lr, device,
-                                      mode, weights)
+                                      mode, weights, loss=loss, loss_scale=loss_scale)
     if optimizer != "lm_rig":
         raise ValueError(f"optimizer must be 'adam', 'lm' or 'lm_rig', got {optimizer!r}")
     if mode not in MODES:
@@ -776,7 +779,7 @@ def run_local_ba(K_torch, R_init_torch, t_init_torch, X3d_init_torch, x2d_torch,
     conf = conf2d_torch.detach().to(dev, torch.float32)
     X0 = X3d_init_torch.detach().to(dev, torch.float32)
     iters = int(max(1, min(int(num_iters), 64)))
-    ba = ba_solve(x2d, conf, K, R0, t0, X0, num_iters=iters, mode=mode, lam0=float(lr))
+    ba = ba_solve(x2d, conf, K, R0, t0, X0, num_iters=iters, mode=mode, lam0=float(lr), loss=loss, loss_scale=loss_scale)
     out_dtype = R_init_torch.dtype
     if mode == "pose_only":   # the cameras are not parameters: hand the caller's back bit for bit
         Rb = R_init_torch.detach() if R.ndim == 4 else R_init_torch.detach()[None].expand(Tn, Cn, 3, 3)

@@ -183,13 +183,19 @@ class RegularisedBundleAdjuster(RegLMSequencer):
     K (C,3,3) | (3,3); R (T,C,3,3) | (C,3,3); t (T,C,3) | (C,3); X0 (T,J,3): tensors or arrays, any float dtype
     mode: "pose_only" (points), "pose_cam_t" (points + every frame's camera translations), "full" (+ rotations)
     group: process group when the clip is sharded by contiguous frame ranges in rank order (None = the default group if
-    torch.distributed is initialised); local_only=True solves this rank's frames alone."""
+    torch.distributed is initialised); local_only=True solves this rank's frames alone.
+    loss: "l2" (default: loss.py's squared pixel error), "huber" or "cauchy" on the reprojection term - a robust M-estimator
+    against gross 2D detector failures (swapped limbs, invented occluded joints), solved by iteratively reweighted
+    Gauss-Newton (include/ska.h); the four regularisers stay squared.  loss_scale: its scale in pixels (required, > 0, for
+    "huber" / "cauchy").  `history` and `cost_value` report the robust cost."""
 
     def __init__(self, x2d, conf, K, R, t, X0, *, mode: str = "pose_only", weights=None, lam0: float = 1e-3, max_iters: int = 64,
                  cg_iters: int = 64, cg_tol: float = 1e-8, check_every: int = 0, group=None, local_only: bool = False,
-                 peer_exchange: bool = True, fuse_exchange: bool = True):
+                 peer_exchange: bool = True, fuse_exchange: bool = True, loss: str = "l2", loss_scale=None):
         if mode not in MODES:
             raise ValueError(f"unknown mode {mode!r}; expected one of {MODES}")
+        self.loss = loss
+        self.loss_id, self.loss_scale = _cabi.check_loss(loss, loss_scale)
         if not (x2d.is_cuda and conf.is_cuda):
             raise RuntimeError("x2d and conf must be CUDA tensors: this package has no CPU path")
         if x2d.dim() != 4 or x2d.shape[-1] != 2:
@@ -311,16 +317,16 @@ class RegularisedBundleAdjuster(RegLMSequencer):
             _lib.check(fn(C.byref(self.prob), *args, _stream_ptr(self.dev)))
 
     def cost(self, which: int):
-        self._call(self.lib.ska_ba_reg_cost_f64, which)
+        self._call(self.lib.ska_ba_reg_cost_robust_f64, which, self.loss_id, self.loss_scale)
 
     def finish_cost(self, which: int):
         self._call(self.lib.ska_ba_reg_finish_cost_f64, which)
 
     def linearize(self):
-        self._call(self.lib.ska_ba_reg_linearize_f64)
+        self._call(self.lib.ska_ba_reg_linearize_robust_f64, self.loss_id, self.loss_scale)
 
     def cg(self, op: int):
-        self._call(self.lib.ska_ba_reg_cg_f64, op)
+        self._call(self.lib.ska_ba_reg_cg_robust_f64, op, self.loss_id, self.loss_scale)
 
     def apply(self):
         self._call(self.lib.ska_ba_reg_apply_f64)
@@ -363,10 +369,11 @@ class RegularisedBundleAdjuster(RegLMSequencer):
 
 
 def run_local_ba_lm(K_torch, R_init_torch, t_init_torch, X3d_init_torch, x2d_torch, conf2d_torch, num_iters=20, lr=1e-3, device="cuda",
-                    mode="pose_only", weights=None, cg_iters=64, cg_tol=1e-8, graph=False, group=None):
+                    mode="pose_only", weights=None, cg_iters=64, cg_tol=1e-8, graph=False, group=None, loss="l2", loss_scale=None):
     """The reference's call (vggt/multi_view_process.py:553-564) answered by LM on the configured objective.  `lr` is the
-    initial damping lambda0 (the one scalar the call site passes to its optimiser).  Returns (R_opt, t_opt, X_opt, history)
-    in X3d_init's dtype; history rows: HIST_KEYS."""
+    initial damping lambda0 (the one scalar the call site passes to its optimiser).  `loss` / `loss_scale`: the reprojection
+    term's loss, as RegularisedBundleAdjuster takes them.  Returns (R_opt, t_opt, X_opt, history) in X3d_init's dtype;
+    history rows: HIST_KEYS."""
     dev = torch.device(device)
     if dev.type != "cuda":
         raise RuntimeError("run_local_ba runs on a CUDA device: this package has no CPU path")
@@ -377,7 +384,7 @@ def run_local_ba_lm(K_torch, R_init_torch, t_init_torch, X3d_init_torch, x2d_tor
     s = RegularisedBundleAdjuster(to32(x2d_torch), to32(conf2d_torch), torch.as_tensor(K_torch).detach(), torch.as_tensor(R_init_torch).detach(),
                                   torch.as_tensor(t_init_torch).detach(), torch.as_tensor(X3d_init_torch).detach(), mode=mode, weights=weights,
                                   lam0=float(lr), max_iters=max(int(num_iters), 1), cg_iters=cg_iters, cg_tol=cg_tol,
-                                  check_every=0 if graph else 8, group=group, local_only=group is None)
+                                  check_every=0 if graph else 8, group=group, local_only=group is None, loss=loss, loss_scale=loss_scale)
     s.run(int(num_iters), graph=graph)
     return s.R.to(dt).clone(), s.t.to(dt).clone(), s.X.to(dt).clone(), s.history
 

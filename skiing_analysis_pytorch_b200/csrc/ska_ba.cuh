@@ -86,6 +86,33 @@ __device__ __forceinline__ void robust_loss(float s, float d, float& rho, float&
   }
 }
 
+// fp64 twin for the regularised LM (ska_ba_reg.cu), split because only its cost kernel needs rho: the scale arrives as
+// d, d^2 and 1/d^2 (computed once on the host), so omega costs Huber one rsqrt and a select and Cauchy one reciprocal.
+// The same s gives the same bits in every kernel that recomputes omega.
+struct RobustScale {
+  double d, d2, id2;
+};
+template <int Loss>
+__device__ __forceinline__ double robust_omega(double s, const RobustScale& r) {
+  if constexpr (Loss == kLossHuber) {
+    return s <= r.d2 ? 1.0 : r.d * rsqrt(s);
+  } else if constexpr (Loss == kLossCauchy) {
+    return 1.0 / (1.0 + s * r.id2);
+  } else {
+    return 1.0;
+  }
+}
+template <int Loss>
+__device__ __forceinline__ double robust_rho(double s, const RobustScale& r) {
+  if constexpr (Loss == kLossHuber) {
+    return s <= r.d2 ? s : 2.0 * r.d * sqrt(s) - r.d2;
+  } else if constexpr (Loss == kLossCauchy) {
+    return r.d2 * log1p(s * r.id2);
+  } else {
+    return s;
+  }
+}
+
 // One observation: residual e, Jacobian rows of (u,v) w.r.t. X_c (ju, jv) and p = R X.
 struct ObsLin {
   float eu, ev;

@@ -19,6 +19,10 @@
 // then ba_reduce_columns.  Nothing synchronises with the host: the CG scalars, the convergence flag, the gain ratio and
 // the accept / reject decision live in d_sc, so a whole LM iteration (with its NCCL all-reduces when sharded) replays
 // as one CUDA graph.
+//
+// Robust loss (Huber / Cauchy, include/ska.h; spec tests/oracle_robust_reg.py run_lm_reg): the kernels that read observations
+// take it as a template argument.  The reprojection weight becomes c_r conf omega(s) in every sum of the step (observe<Loss>)
+// and the cost sums conf rho(s); the regularisers and every other kernel are the L2 solver's.
 #include <cuda_runtime.h>
 #include <math.h>
 
@@ -64,6 +68,12 @@ struct RegArgs {
   double* ppart;  // [W]  predicted-decrease partials (apply -> cost(trial))
   int W;
 };
+// The robust scale goes after everything the L2 solver passes a kernel, so that the L2 instantiations read every parameter
+// at its old offset: appended to the argument block of the kernels that take nothing else (linearisation, matrix-vector
+// product), a trailing parameter of reg_cost_kernel and reg_precond_kernel.
+struct RegArgsRs : RegArgs {
+  RobustScale rs;
+};
 
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll
@@ -92,7 +102,10 @@ __device__ __forceinline__ void sym3vec(const double N[6], const double v[3], do
   o[2] = N[2] * v[0] + N[4] * v[1] + N[5] * v[2];
 }
 
-// One observation: camera-frame point, residual, N = w (ju ju^T + jv jv^T), q = w (ju eu + jv ev).  loss.py:17-87.
+// One observation: camera-frame point, residual, N = w' (ju ju^T + jv jv^T), q = w' (ju eu + jv ev).  loss.py:17-87.
+// w' = w under L2; under a robust loss w' = w omega(|e|^2), omega at the current state and not differentiated (iteratively
+// reweighted Gauss-Newton).  Every kernel that needs N recomputes omega from the same d2 expression, so the linearisation,
+// the matrix-vector product and the preconditioner of a trial weight each observation with the same bits.
 struct Obs {
   double p[3];  // R X
   double N[6];
@@ -100,8 +113,9 @@ struct Obs {
   double d2;    // |e|^2
   bool clamped;
 };
+template <int Loss>
 __device__ __forceinline__ void observe(const double* cam /*R(9) t(3)*/, const double* K, const double X[3], double u_obs, double v_obs,
-                                        double w, Obs& o) {
+                                        double w, const RobustScale& rs, Obs& o) {
   matvec3(cam, X, o.p);
   const double xc = o.p[0] + cam[9], yc = o.p[1] + cam[10], zc = o.p[2] + cam[11];
   o.clamped = zc < kZMin;
@@ -112,6 +126,7 @@ __device__ __forceinline__ void observe(const double* cam /*R(9) t(3)*/, const d
   const double ju[3] = {K[0] * iz, K[1] * iz, -(K[0] * x + K[1] * y) * iz * live};
   const double jv[3] = {K[3] * iz, K[4] * iz, -(K[3] * x + K[4] * y) * iz * live};
   o.d2 = eu * eu + ev * ev;
+  if constexpr (Loss != kLossL2) w *= robust_omega<Loss>(o.d2, rs);
   o.N[0] = w * (ju[0] * ju[0] + jv[0] * jv[0]);
   o.N[1] = w * (ju[0] * ju[1] + jv[0] * jv[1]);
   o.N[2] = w * (ju[0] * ju[2] + jv[0] * jv[2]);
@@ -175,7 +190,8 @@ __device__ __forceinline__ const double* frame_C(const RegArgs& a, int buf, int6
 // ------------------------------------------------------------------------------------------------ cost
 // sums of one point (buffer `buf`): raw reprojection sum, clamp count, temporal / smoothness pairs (t, t+1) owned by t,
 // per-bone sum L and sum L^2, baseline sum b and sum b^2.  The weights and the means enter in reg_finish_cost.
-__global__ void __launch_bounds__(32 * kWarpsPerBlock) reg_cost_kernel(const RegArgs a, int which) {
+template <int Loss>
+__global__ void __launch_bounds__(32 * kWarpsPerBlock) reg_cost_kernel(const RegArgs a, int which, const RobustScale rs) {
   const int lane = threadIdx.x & 31, wid = blockIdx.x * kWarpsPerBlock + (threadIdx.x >> 5);
   const int buf = which == 0 ? (int)a.sc[SC_CUR] : 1 - (int)a.sc[SC_CUR];
   double s_rep = 0.0, s_cl = 0.0, s_tmp = 0.0, s_sm = 0.0, s_b = 0.0, s_b2 = 0.0, s_L = 0.0, s_L2 = 0.0;
@@ -190,8 +206,8 @@ __global__ void __launch_bounds__(32 * kWarpsPerBlock) reg_cost_kernel(const Reg
         const float2 uv = *reinterpret_cast<const float2*>(a.x2d + ((f * a.C + c) * a.J + j) * 2);
         const double w = (double)a.conf[(f * a.C + c) * a.J + j];
         Obs o;
-        observe(Cm + 12 * c, a.K + 9 * c, Xj, (double)uv.x, (double)uv.y, 1.0, o);
-        s_rep += w * o.d2;
+        observe<kLossL2>(Cm + 12 * c, a.K + 9 * c, Xj, (double)uv.x, (double)uv.y, 1.0, rs, o);
+        s_rep += w * robust_rho<Loss>(o.d2, rs);
         s_cl += o.clamped ? 1.0 : 0.0;
       }
       if (next) {
@@ -304,7 +320,8 @@ __device__ __forceinline__ int up6(int r, int c) { return r * 6 - r * (r - 1) / 
 // ------------------------------------------------------------------------------------------------ linearisation
 // per frame: gradient g = J^T r, D = diag(J^T J), r_cg = -g, the damped point blocks' inverses, and the Cholesky factor of
 // the frame's Schur complement S = Dc - sum_j W_j^T Dp_j^-1 W_j  (Dp, Dc: damped diagonal blocks of J^T J).
-__global__ void __launch_bounds__(32 * kWarpsPerBlock, 4) reg_linearize_kernel(const RegArgs a) {
+template <int Loss>
+__global__ void __launch_bounds__(32 * kWarpsPerBlock, 4) reg_linearize_kernel(const RegArgsRs a) {
   extern __shared__ double smem_d[];
   // launched with 4, 2 or 1 warps per block (the largest frames - 96 joints x 8 cameras - need 60 KB of shared memory per warp)
   const int lane = threadIdx.x & 31, wl = threadIdx.x >> 5, wid = blockIdx.x * (int)(blockDim.x >> 5) + wl;
@@ -337,7 +354,7 @@ __global__ void __launch_bounds__(32 * kWarpsPerBlock, 4) reg_linearize_kernel(c
         const float2 uv = *reinterpret_cast<const float2*>(a.x2d + ((f * a.C + c) * a.J + j) * 2);
         const double w = cr * (double)a.conf[(f * a.C + c) * a.J + j];
         Obs o;
-        observe(cam, K, sm.X + 3 * j, (double)uv.x, (double)uv.y, w, o);
+        observe<Loss>(cam, K, sm.X + 3 * j, (double)uv.x, (double)uv.y, w, a.rs, o);
         // Hpp += R^T N R, gX += R^T q
         double RtN[3][3];  // rows of R^T N: (R^T N)[i][k] = sum_a R[a][i] N[a][k]
 #pragma unroll
@@ -512,7 +529,7 @@ __global__ void __launch_bounds__(32 * kWarpsPerBlock, 4) reg_linearize_kernel(c
           const float2 uv = *reinterpret_cast<const float2*>(a.x2d + ((f * a.C + c) * a.J + j) * 2);
           const double w = cr * (double)a.conf[(f * a.C + c) * a.J + j];
           Obs o;
-          observe(cam, a.K + 9 * c, sm.X + 3 * j, (double)uv.x, (double)uv.y, w, o);
+          observe<Loss>(cam, a.K + 9 * c, sm.X + 3 * j, (double)uv.x, (double)uv.y, w, a.rs, o);
 #pragma unroll
           for (int k = 0; k < 6; ++k) {
             double col[3] = {0.0, 0.0, 0.0};
@@ -571,7 +588,8 @@ __global__ void __launch_bounds__(32 * kWarpsPerBlock, 4) reg_linearize_kernel(c
 
 // ------------------------------------------------------------------------------------------------ matrix-vector product
 // y = (J^T J + lam D) p for the frame's row; partial dot p . y
-__global__ void __launch_bounds__(32 * kWarpsPerBlock, 4) reg_matvec_kernel(const RegArgs a) {
+template <int Loss>
+__global__ void __launch_bounds__(32 * kWarpsPerBlock, 4) reg_matvec_kernel(const RegArgsRs a) {
   extern __shared__ double smem_d[];
   const int lane = threadIdx.x & 31, wl = threadIdx.x >> 5, wid = blockIdx.x * kWarpsPerBlock + wl;
   const double* sc = a.sc;
@@ -608,7 +626,7 @@ __global__ void __launch_bounds__(32 * kWarpsPerBlock, 4) reg_matvec_kernel(cons
           const float2 uv = *reinterpret_cast<const float2*>(a.x2d + ((f * a.C + c) * a.J + j) * 2);
           const double w = cr * (double)a.conf[(f * a.C + c) * a.J + j];
           Obs o;
-          observe(cam, a.K + 9 * c, sX + 3 * j, (double)uv.x, (double)uv.y, w, o);
+          observe<Loss>(cam, a.K + 9 * c, sX + 3 * j, (double)uv.x, (double)uv.y, w, a.rs, o);
           double dxc[3];
           matvec3(cam, V + 3 * j, dxc);  // R pX
           if (cams_free) {
@@ -723,7 +741,8 @@ __global__ void __launch_bounds__(32 * kWarpsPerBlock, 4) reg_matvec_kernel(cons
 
 // ------------------------------------------------------------------------------------------------ CG update + preconditioner
 // x += alpha p, r -= alpha y, z = M^-1 r (the frame's system through its Schur complement); partial dot r . z
-__global__ void __launch_bounds__(32 * kWarpsPerBlock, 4) reg_precond_kernel(const RegArgs a, int first) {
+template <int Loss>
+__global__ void __launch_bounds__(32 * kWarpsPerBlock, 4) reg_precond_kernel(const RegArgs a, int first, const RobustScale rs) {
   extern __shared__ double smem_d[];
   const int lane = threadIdx.x & 31, wl = threadIdx.x >> 5, wid = blockIdx.x * kWarpsPerBlock + wl;
   const double* sc = a.sc;
@@ -786,7 +805,7 @@ __global__ void __launch_bounds__(32 * kWarpsPerBlock, 4) reg_precond_kernel(con
           const float2 uv = *reinterpret_cast<const float2*>(a.x2d + ((f * a.C + c) * a.J + j) * 2);
           const double w = cr * (double)a.conf[(f * a.C + c) * a.J + j];
           Obs o;
-          observe(cam, a.K + 9 * c, sX + 3 * j, (double)uv.x, (double)uv.y, w, o);
+          observe<Loss>(cam, a.K + 9 * c, sX + 3 * j, (double)uv.x, (double)uv.y, w, rs, o);
           double ru[3], nb[3], pw[3];
           matvec3(cam, U + 3 * j, ru);
           sym3vec(o.N, ru, nb);
@@ -824,7 +843,7 @@ __global__ void __launch_bounds__(32 * kWarpsPerBlock, 4) reg_precond_kernel(con
           const float2 uv = *reinterpret_cast<const float2*>(a.x2d + ((f * a.C + c) * a.J + j) * 2);
           const double w = cr * (double)a.conf[(f * a.C + c) * a.J + j];
           Obs o;
-          observe(cam, a.K + 9 * c, sX + 3 * j, (double)uv.x, (double)uv.y, w, o);
+          observe<Loss>(cam, a.K + 9 * c, sX + 3 * j, (double)uv.x, (double)uv.y, w, rs, o);
           const double* zc = B + 6 * c;
           double cx[3];
           cross(zc, o.p, cx);
@@ -998,7 +1017,8 @@ __device__ __forceinline__ double block_sum_to(double v, double* sh) {
   return t;
 }
 
-__global__ void __launch_bounds__(kPtBlock) reg_pt_linearize_kernel(const RegArgs a) {
+template <int Loss>
+__global__ void __launch_bounds__(kPtBlock) reg_pt_linearize_kernel(const RegArgsRs a) {
   const double* sc = a.sc;
   const int buf = (int)sc[SC_CUR];
   const double lam = sc[SC_LAM], cr = sc[SC_CR], cl = sc[SC_CL], ct = sc[SC_CT];
@@ -1017,7 +1037,7 @@ __global__ void __launch_bounds__(kPtBlock) reg_pt_linearize_kernel(const RegArg
       const float2 uv = *reinterpret_cast<const float2*>(a.x2d + ((f * a.C + c) * a.J + j) * 2);
       const double w = cr * (double)a.conf[(f * a.C + c) * a.J + j];
       Obs o;
-      observe(cam, a.K + 9 * c, Xj, (double)uv.x, (double)uv.y, w, o);
+      observe<Loss>(cam, a.K + 9 * c, Xj, (double)uv.x, (double)uv.y, w, a.rs, o);
       double RtN[3][3];
 #pragma unroll
       for (int r = 0; r < 3; ++r) {
@@ -1073,7 +1093,8 @@ __global__ void __launch_bounds__(kPtBlock) reg_pt_linearize_kernel(const RegArg
   }
 }
 
-__global__ void __launch_bounds__(kPtBlock) reg_pt_matvec_kernel(const RegArgs a) {
+template <int Loss>
+__global__ void __launch_bounds__(kPtBlock) reg_pt_matvec_kernel(const RegArgsRs a) {
   __shared__ double sh[kPtBlock / 32];
   const double* sc = a.sc;
   double dot = 0.0;
@@ -1097,7 +1118,7 @@ __global__ void __launch_bounds__(kPtBlock) reg_pt_matvec_kernel(const RegArgs a
         const float2 uv = *reinterpret_cast<const float2*>(a.x2d + ((f * a.C + c) * a.J + j) * 2);
         const double w = cr * (double)a.conf[(f * a.C + c) * a.J + j];
         Obs o;
-        observe(cam, a.K + 9 * c, Xj, (double)uv.x, (double)uv.y, w, o);
+        observe<Loss>(cam, a.K + 9 * c, Xj, (double)uv.x, (double)uv.y, w, a.rs, o);
         double dxc[3], nq[3], back[3];
         matvec3(cam, pj, dxc);
         sym3vec(o.N, dxc, nq);
@@ -1233,15 +1254,27 @@ static int set_smem(Kern kern, size_t bytes) {
   return SKA_OK;
 }
 
+// The instantiation of a loss-templated kernel for `loss` (SKA_BA_LOSS_*, validated by the C ABI).  The launch sites bind
+// it to a local pointer of the kernel's own name, so that every loss runs through the same launch code.
+template <typename Kern>
+static Kern by_loss(int loss, Kern l2, Kern huber, Kern cauchy) {
+  return loss == SKA_BA_LOSS_HUBER ? huber : loss == SKA_BA_LOSS_CAUCHY ? cauchy : l2;
+}
+#define SKA_REG_BY_LOSS(kern) by_loss(loss, ska::kern<kLossL2>, ska::kern<kLossHuber>, ska::kern<kLossCauchy>)
+
+static RobustScale robust_scale(double d) { return RobustScale{d, d * d, d > 0.0 ? 1.0 / (d * d) : 0.0}; }
+
 }  // namespace
 
 size_t ba_reg_workspace_bytes(int64_t T_local) { return (size_t)grid_blocks(T_local) * kWarpsPerBlock * (NS + 2) * sizeof(double); }
 
-int ba_reg_cost(const SkaBaRegProblem& p, int which, cudaStream_t s) {
+int ba_reg_cost(const SkaBaRegProblem& p, int which, int loss, double loss_scale, cudaStream_t s) {
   RegArgs a;
   int rc = fill(p, a);
   if (rc != SKA_OK) return rc;
-  reg_cost_kernel<<<a.W / kWarpsPerBlock, 32 * kWarpsPerBlock, 0, s>>>(a, which);
+  const RobustScale rs = robust_scale(loss_scale);
+  const auto reg_cost_kernel = SKA_REG_BY_LOSS(reg_cost_kernel);
+  reg_cost_kernel<<<a.W / kWarpsPerBlock, 32 * kWarpsPerBlock, 0, s>>>(a, which, rs);
   if ((rc = check_launch()) != SKA_OK) return rc;
   if ((rc = launch_reduce(a.part, a.W, NS, a.sums + (which ? NS : 0), s)) != SKA_OK) return rc;
   if (which) rc = launch_reduce(a.ppart, a.W, 1, a.sums + NS + SUM_PRED, s);
@@ -1264,11 +1297,13 @@ int ba_reg_finish_cost(const SkaBaRegProblem& p, int which, cudaStream_t s) {
   return check_launch();
 }
 
-int ba_reg_linearize(const SkaBaRegProblem& p, cudaStream_t s) {
-  RegArgs a;
+int ba_reg_linearize(const SkaBaRegProblem& p, int loss, double loss_scale, cudaStream_t s) {
+  RegArgsRs a;
   int rc = fill(p, a);
   if (rc != SKA_OK) return rc;
+  a.rs = robust_scale(loss_scale);
   if (a.free6 == 0) {  // points only: one thread per point
+    const auto reg_pt_linearize_kernel = SKA_REG_BY_LOSS(reg_pt_linearize_kernel);
     reg_pt_linearize_kernel<<<pt_grid(a), kPtBlock, 0, s>>>(a);
     return check_launch();
   }
@@ -1276,15 +1311,20 @@ int ba_reg_linearize(const SkaBaRegProblem& p, cudaStream_t s) {
   int wpb = kWarpsPerBlock;
   while (wpb > 1 && per_warp * wpb > (size_t)227 * 1024) wpb /= 2;
   const size_t bytes = per_warp * wpb;
+  const auto reg_linearize_kernel = SKA_REG_BY_LOSS(reg_linearize_kernel);
   if ((rc = set_smem(reg_linearize_kernel, bytes)) != SKA_OK) return rc;
   reg_linearize_kernel<<<a.W / wpb, 32 * wpb, bytes, s>>>(a);
   return check_launch();
 }
 
-int ba_reg_cg(const SkaBaRegProblem& p, int op, cudaStream_t s) {
-  RegArgs a;
+int ba_reg_cg(const SkaBaRegProblem& p, int op, int loss, double loss_scale, cudaStream_t s) {
+  RegArgsRs a;
   int rc = fill(p, a);
   if (rc != SKA_OK) return rc;
+  a.rs = robust_scale(loss_scale);  // read by MATVEC, and by BEGIN / UPDATE with free cameras: the ops that read observations
+  const auto reg_precond_kernel = SKA_REG_BY_LOSS(reg_precond_kernel);
+  const auto reg_matvec_kernel = SKA_REG_BY_LOSS(reg_matvec_kernel);
+  const auto reg_pt_matvec_kernel = SKA_REG_BY_LOSS(reg_pt_matvec_kernel);
   const int blocks = a.W / kWarpsPerBlock;
   switch (op) {
     case SKA_BA_REG_CG_BEGIN:
@@ -1309,7 +1349,7 @@ int ba_reg_cg(const SkaBaRegProblem& p, int op, cudaStream_t s) {
         if (ce == cudaSuccess) ce = cudaMemsetAsync(a.y, 0, n, s);
         if (ce != cudaSuccess) return set_error((int)ce, cudaGetErrorString(ce));
       }
-      reg_precond_kernel<<<blocks, 32 * kWarpsPerBlock, bytes, s>>>(a, op == SKA_BA_REG_CG_BEGIN ? 1 : 0);
+      reg_precond_kernel<<<blocks, 32 * kWarpsPerBlock, bytes, s>>>(a, op == SKA_BA_REG_CG_BEGIN ? 1 : 0, a.rs);
       if ((rc = check_launch()) != SKA_OK) return rc;
       return launch_reduce(a.dpart, a.W, 1, a.sc + SC_DOT, s);
     }
@@ -1366,5 +1406,7 @@ int ba_reg_control(const SkaBaRegProblem& p, cudaStream_t s) {
   reg_control_kernel<<<1, 32, 0, s>>>(a, p.d_hist, p.hist_rows);
   return check_launch();
 }
+
+#undef SKA_REG_BY_LOSS
 
 }  // namespace ska

@@ -294,12 +294,33 @@ size_t ska_ba_reg_workspace_bytes(int64_t T_local) { return T_local < 1 ? 0 : ba
 #define SKA_REG_ENTRY(call)                                                        \
   if (p == nullptr) return set_error(SKA_EINVAL, "problem pointer must not be NULL"); \
   return call
-int ska_ba_reg_cost_f64(const SkaBaRegProblem* p, int32_t which, void* stream) { SKA_REG_ENTRY(ba_reg_cost(*p, which, (cudaStream_t)stream)); }
+// the regularised LM's kernels are fp64: a robust scale needs a finite d > 0 whose square is a normal fp64 number
+static int check_reg_loss(int32_t loss, double loss_scale) {
+  if (loss != SKA_BA_LOSS_L2 && loss != SKA_BA_LOSS_HUBER && loss != SKA_BA_LOSS_CAUCHY) return set_error(SKA_EINVAL, "unknown loss");
+  if (loss != SKA_BA_LOSS_L2 && !(isfinite(loss_scale) && loss_scale > 0.0 && isfinite(loss_scale * loss_scale) && loss_scale * loss_scale >= DBL_MIN))
+    return set_error(SKA_EINVAL, "a robust loss needs a finite loss_scale > 0 whose square is a normal fp64 number");
+  return SKA_OK;
+}
+#define SKA_REG_LOSS_ENTRY(call)                                                        \
+  if (p == nullptr) return set_error(SKA_EINVAL, "problem pointer must not be NULL");   \
+  if (const int rc = check_reg_loss(loss, loss_scale); rc != SKA_OK) return rc;        \
+  return call
+int ska_ba_reg_cost_robust_f64(const SkaBaRegProblem* p, int32_t which, int32_t loss, double loss_scale, void* stream) {
+  SKA_REG_LOSS_ENTRY(ba_reg_cost(*p, which, loss, loss_scale, (cudaStream_t)stream));
+}
+int ska_ba_reg_linearize_robust_f64(const SkaBaRegProblem* p, int32_t loss, double loss_scale, void* stream) {
+  SKA_REG_LOSS_ENTRY(ba_reg_linearize(*p, loss, loss_scale, (cudaStream_t)stream));
+}
+int ska_ba_reg_cg_robust_f64(const SkaBaRegProblem* p, int32_t op, int32_t loss, double loss_scale, void* stream) {
+  SKA_REG_LOSS_ENTRY(ba_reg_cg(*p, op, loss, loss_scale, (cudaStream_t)stream));
+}
+#undef SKA_REG_LOSS_ENTRY
+int ska_ba_reg_cost_f64(const SkaBaRegProblem* p, int32_t which, void* stream) { return ska_ba_reg_cost_robust_f64(p, which, SKA_BA_LOSS_L2, 0.0, stream); }
 int ska_ba_reg_finish_cost_f64(const SkaBaRegProblem* p, int32_t which, void* stream) {
   SKA_REG_ENTRY(ba_reg_finish_cost(*p, which, (cudaStream_t)stream));
 }
-int ska_ba_reg_linearize_f64(const SkaBaRegProblem* p, void* stream) { SKA_REG_ENTRY(ba_reg_linearize(*p, (cudaStream_t)stream)); }
-int ska_ba_reg_cg_f64(const SkaBaRegProblem* p, int32_t op, void* stream) { SKA_REG_ENTRY(ba_reg_cg(*p, op, (cudaStream_t)stream)); }
+int ska_ba_reg_linearize_f64(const SkaBaRegProblem* p, void* stream) { return ska_ba_reg_linearize_robust_f64(p, SKA_BA_LOSS_L2, 0.0, stream); }
+int ska_ba_reg_cg_f64(const SkaBaRegProblem* p, int32_t op, void* stream) { return ska_ba_reg_cg_robust_f64(p, op, SKA_BA_LOSS_L2, 0.0, stream); }
 int ska_ba_reg_apply_f64(const SkaBaRegProblem* p, void* stream) { SKA_REG_ENTRY(ba_reg_apply(*p, (cudaStream_t)stream)); }
 int ska_ba_reg_control_f64(const SkaBaRegProblem* p, void* stream) { SKA_REG_ENTRY(ba_reg_control(*p, (cudaStream_t)stream)); }
 #undef SKA_REG_ENTRY

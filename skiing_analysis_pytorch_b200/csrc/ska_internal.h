@@ -55,10 +55,10 @@ int ba_calib_control(int C, const double* red, double* red2, double* cams, doubl
 
 // regularised LM over the full configured objective, per-frame cameras (ska_ba_reg.cu)
 size_t ba_reg_workspace_bytes(int64_t T_local);
-int ba_reg_cost(const SkaBaRegProblem& p, int which, cudaStream_t s);
+int ba_reg_cost(const SkaBaRegProblem& p, int which, int loss, double loss_scale, cudaStream_t s);
 int ba_reg_finish_cost(const SkaBaRegProblem& p, int which, cudaStream_t s);
-int ba_reg_linearize(const SkaBaRegProblem& p, cudaStream_t s);
-int ba_reg_cg(const SkaBaRegProblem& p, int op, cudaStream_t s);
+int ba_reg_linearize(const SkaBaRegProblem& p, int loss, double loss_scale, cudaStream_t s);
+int ba_reg_cg(const SkaBaRegProblem& p, int op, int loss, double loss_scale, cudaStream_t s);
 int ba_reg_apply(const SkaBaRegProblem& p, cudaStream_t s);
 int ba_reg_control(const SkaBaRegProblem& p, cudaStream_t s);
 // exchange over NVLink peer memory (ska_peer.cu)
